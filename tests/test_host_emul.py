@@ -19,17 +19,14 @@ from ray_tracing_series_rust_b200 import capi
 import parity_utils as pu
 
 HERE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "host_emul")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _build_emul(name, extra=()):
-    so = os.path.join(HERE, name)
-    srcs = [os.path.join(HERE, "emul.cpp"), os.path.join(HERE, "cuda_shim.h"),
-            os.path.join(ROOT, "ray_tracing_series_rust_b200", "csrc", "cuda", "rt_device.cuh"),
-            os.path.join(ROOT, "ray_tracing_series_rust_b200", "csrc", "rt_types.h")]
-    if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
-        subprocess.check_call(["g++", "-std=c++17", "-O2", "-fPIC", "-shared", "-ffp-contract=off", "-Wno-unknown-pragmas", *extra,
-                               "-I/usr/local/cuda/include", srcs[0], "-o", so])
+def _build_emul(so, extra=()):
+    """Compiles emul.cpp to `so`, a fresh path of this test session: a library kept between sessions could predate a change to
+    any header emul.cpp includes, and parallel test workers must not write one file at once."""
+    cuda_include = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "include")
+    subprocess.check_call(["g++", "-std=c++17", "-O2", "-fPIC", "-shared", "-ffp-contract=off", "-Wno-unknown-pragmas", *extra,
+                           "-I" + cuda_include, os.path.join(HERE, "emul.cpp"), "-o", so])
     lib = C.CDLL(so)
     lib.emul_sizeof_device_scene.restype = C.c_uint64
     lib.emul_trace_batch.restype = C.c_int32
@@ -44,8 +41,8 @@ def _build_emul(name, extra=()):
 
 
 @pytest.fixture(scope="module")
-def emul():
-    return _build_emul("libemul.so")
+def emul(tmp_path_factory):
+    return _build_emul(str(tmp_path_factory.mktemp("emul") / "libemul.so"))
 
 
 def host_scene(emul, scene_id, seed=0xB001, param=0, width=2):
