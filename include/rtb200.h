@@ -267,6 +267,26 @@ RTB_EXPORT int32_t rt_render_multi(rt_scene* s, const rt_render_config* cfg, int
                                    double* out_screen, int64_t* out_accum, rt_stats* stats);
 /* rt_scene_commit + upload of the flattened scene to GPUs 1..n_gpus-1 (otherwise the first rt_render_multi does it). */
 RTB_EXPORT int32_t rt_scene_commit_multi(rt_scene* s, int32_t n_gpus);
+
+/* Adaptive sampling: every pixel is rendered until its noise estimate converges, at most cfg->samples_per_pixel (= max) samples.
+ * Round k traces samples [k*step, min((k+1)*step, max)) of the pixels still active, alternately into two half accumulators A
+ * (even k) and B (odd k).  After every odd round, at n = (k+1)*step samples with min_samples <= n < max, each active pixel's
+ * error is computed in f64 from its int64 sums (h = n/2 samples in each half, S = h * 2^32):
+ *     err = (((|a_r-b_r| + |a_g-b_g|) + |a_b-b_b|) / S) / sqrt(1e-4 + (((a_r+b_r) + (a_g+b_g)) + (a_b+b_b)) / (2*S))
+ * A pixel stays active iff a pixel with !(err < threshold) lies within Chebyshev distance `radius` of it (on a rendered row);
+ * a pixel that leaves keeps n samples, one that never leaves gets max.  Path ids are rt_render's (pixel * max + sample), so a
+ * pixel's sums are exactly those of rt_render over its own samples: threshold 0 reproduces rt_render bit for bit.
+ * out_accum = A + B; out_screen resolves each pixel with its own count; out_samples (W*H int32, nullable) = the counts, 0 on
+ * unrendered compat_threads rows.  cfg must render the whole [0, samples_per_pixel), without a tile shard (RT_RENDER_TILE_SHARD
+ * with count > 1; count 0 or 1 means no sharding, as in rt_render) and without RT_RENDER_NO_WAIT; the mode flags apply to every round.  stats: counters and ms_device summed over the rounds. */
+typedef struct rt_adaptive_config {
+    int32_t min_samples; /* 0 .. samples_per_pixel: no pixel stops before this many samples */
+    int32_t step;        /* >= 1: samples per round; check points every 2 rounds */
+    double threshold;    /* >= 0 and finite; 0 = no pixel converges (result == rt_render) */
+    int32_t radius;      /* 0..8: a pixel stays active while an unconverged pixel is this close */
+} rt_adaptive_config;
+RTB_EXPORT int32_t rt_render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac,
+                                      double* out_screen, int64_t* out_accum, int32_t* out_samples, rt_stats* stats);
 #endif
 /* image height the config implies: (image_width as f64 / aspect_ratio) as i32 */
 RTB_EXPORT int32_t RTB_FN(image_height)(const rt_render_config* cfg);

@@ -45,6 +45,15 @@ pub struct RtRenderConfig {
     pub flags: i32,
 }
 
+/// rt_adaptive_config (include/rtb200.h): per-pixel sample counts for rt_render_adaptive
+#[repr(C)]
+pub struct RtAdaptiveConfig {
+    pub min_samples: i32, // 0 ..= samples_per_pixel: no pixel stops before this many samples
+    pub step: i32,        // >= 1: samples per round; check points every 2 rounds
+    pub threshold: f64,   // >= 0 and finite; 0 = no pixel converges (result == rt_render)
+    pub radius: i32,      // 0..=8: a pixel stays active while an unconverged pixel is this close
+}
+
 #[link(name = "rtb200")]
 extern "C" {
     fn rt_scene_create() -> *mut RtScene;
@@ -82,6 +91,9 @@ extern "C" {
     fn rt_render(s: *mut RtScene, cfg: *const RtRenderConfig, out_screen: *mut f64, out_accum: *mut i64, stats: *mut u8) -> i32;
     /// one host thread, n_gpus devices of the box: shards rendered per GPU, summed + resolved over NVLink peer memory (include/rtb200.h)
     fn rt_render_multi(s: *mut RtScene, cfg: *const RtRenderConfig, n_gpus: i32, shard_mode: i32, out_screen: *mut f64, out_accum: *mut i64, stats: *mut u8) -> i32;
+    /// every pixel until its noise estimate converges, at most cfg.samples_per_pixel; out_samples = W*H per-pixel counts (nullable)
+    fn rt_render_adaptive(s: *mut RtScene, cfg: *const RtRenderConfig, ac: *const RtAdaptiveConfig, out_screen: *mut f64, out_accum: *mut i64,
+                          out_samples: *mut i32, stats: *mut u8) -> i32;
     fn rt_render_scene_with_time(s: *mut RtScene, t0: f64, t1: f64, path: *const c_char, cfg: *const RtRenderConfig, out_screen: *mut f64, stats: *mut u8) -> i32;
     fn rt_write_ppm(path: *const c_char, screen: *const f64, w: i32, h: i32) -> i32;
 }

@@ -11,7 +11,8 @@ not the loop around it (its `/video_testing/` driver is absent from the repo), a
                       summed into the int64 accumulator, with an atomic single-file checkpoint every few chunks.  Philox
                       streams are keyed by the global sample index and the sum is integer, so a render that
                       was interrupted and resumed is bit-identical to the one-shot render.
-* `resolve_accumulator`  host mirror of `k_resolve` (Vec3::get_normalized_color, src/vec3.rs:89-107).
+* `resolve_accumulator`  host mirror of `k_resolve` (Vec3::get_normalized_color, src/vec3.rs:89-107), also with per-pixel
+                         sample counts (`k_resolve_adaptive`).
 """
 from __future__ import annotations
 
@@ -24,11 +25,19 @@ import numpy as np
 from . import capi, sharding
 
 
-def resolve_accumulator(accum: np.ndarray, spp: int, rendered_rows: Optional[int] = None) -> np.ndarray:
-    """int64 fixed-point (2^32) radiance sums [H, W, 3] -> the reference's Screen (integer-valued f64, row 0 = bottom)."""
+def resolve_accumulator(accum: np.ndarray, spp, rendered_rows: Optional[int] = None) -> np.ndarray:
+    """int64 fixed-point (2^32) radiance sums [H, W, 3] -> the reference's Screen (integer-valued f64, row 0 = bottom).
+
+    `spp` is one sample count for every pixel, or per-pixel counts [H, W] (rt_render_adaptive's samples; a pixel with 0 samples
+    resolves to black)."""
     s = accum.astype(np.float64) * (1.0 / 4294967296.0)
+    if np.ndim(spp) == 0:
+        scale = 1.0 / float(spp)
+    else:
+        with np.errstate(divide="ignore"):
+            scale = (1.0 / np.asarray(spp, dtype=np.float64))[..., None]
     with np.errstate(invalid="ignore"):
-        c = np.sqrt(s * (1.0 / float(spp)))
+        c = np.sqrt(s * scale)
     c = np.where(c < 0.0, 0.0, np.where(c > 1.0, 1.0, c))  # mutil.rs:1-9
     q = 255.9 * c
     out = np.where(np.isnan(q), 0.0, np.trunc(q))          # `as i32`

@@ -64,9 +64,10 @@ struct JobDev {
     uint32_t n_slots;
     int32_t count_events;
     uint32_t wait_thresh; // k_mega_r: finished lanes that end a traversal round
-    uint32_t tile_rank, tile_count; // RT_RENDER_TILE_SHARD: npix_rendered counts this shard's pixels only
+    uint32_t tile_rank, tile_count; // RT_RENDER_TILE_SHARD: npix_rendered counts this shard's pixels only; tile_count 0 = a pixel list
     uint32_t chunk;                 // fused kernels: consecutive path indices a warp claims per atomic
     unsigned long long path_base;   // this call renders the path indices [path_base, path_base + total_paths) of the sample-major enumeration
+    const uint32_t* pix_list;       // rt_render_adaptive: dense index -> pixel of the active list (npix_rendered entries); null = no list
 };
 
 // Path-state chunks are streamed (read once / written once per kernel): evict-first hints keep them from
@@ -131,8 +132,11 @@ __global__ void k_init(PathState P, Queues Q, uint32_t n) {
 
 // Tile sharding: the shard's pixels are enumerated densely (local row lr = band lr / 4 of this rank, line lr % 4);
 // the global pixel index (accumulator address, Philox path id) is that of the unsharded image.
+// A pixel list (adaptive sampling, tile_count 0) maps the dense index through the list instead.  The whole image (tile_count 1)
+// stays one compare, as before the list existed.
 RT_DEV uint32_t shard_pixel(const JobDev& J, uint32_t q) {
-    if (J.tile_count <= 1u) return q;
+    if (J.tile_count == 1u) return q;
+    if (J.tile_count == 0u) return __ldg(J.pix_list + q);
     const uint32_t W = (uint32_t)J.W, lr = q / W, x = q - lr * W;
     const uint32_t band = (lr / RT_TILE_ROWS) * J.tile_count + J.tile_rank;
     return (band * RT_TILE_ROWS + lr % RT_TILE_ROWS) * W + x;
@@ -1405,6 +1409,8 @@ cudaError_t launch_render(const DeviceScene& scene, const RenderJob& job, const 
             local_rows += std::min<uint32_t>(RT_TILE_ROWS, (uint32_t)job.rows - b * RT_TILE_ROWS);
     }
     J.npix_rendered = (uint32_t)job.width * local_rows;
+    J.pix_list = job.d_pixels;
+    if (job.d_pixels) { J.npix_rendered = job.n_pixels; J.tile_count = 0; } // the caller never combines a list with tile sharding
     J.total_paths = (unsigned long long)J.npix_rendered * (unsigned long long)(job.sample_end - job.sample_begin);
     J.path_base = 0;
     if (job.path_end > job.path_begin) { // a path-range shard of [sample_begin, sample_end): whole samples plus a partial first / last one

@@ -20,6 +20,10 @@ struct RenderJob {
     // rt_render_device_paths: only the path indices [path_begin, path_end) of the call's (pixels x samples) in sample-major order
     // (index = sample * pixels + pixel); 0, 0 = all of them
     uint64_t path_begin = 0, path_end = 0;
+    // rt_render_adaptive: render only the n_pixels pixels of this device list (ascending global pixel indices) instead of the rows
+    // [0, rows); path index = sample * n_pixels + list position.  null = every pixel of [0, rows)
+    const uint32_t* d_pixels = nullptr;
+    uint32_t n_pixels = 0;
 };
 
 #define RT_MODE_WAVEFRONT 0 // k_extend + k_shade_all per iteration, per-material queues, path state in HBM
@@ -70,6 +74,34 @@ cudaError_t launch_flag_publish(uint32_t* flag, uint32_t value, cudaStream_t str
 cudaError_t launch_flag_wait(const uint32_t* flag, uint32_t need, uint32_t* timeout_flag, cudaStream_t stream);
 cudaError_t launch_reduce_resolve(const AccumShards& shards, int64_t* d_sum_out, uint8_t* d_screen_u8, double* d_screen_f64, int32_t W, int32_t H, int32_t spp,
                                   int32_t rows, cudaStream_t stream);
+
+// ---- adaptive sampling (adaptive.cu, rt_render_adaptive)
+// Check point after n samples (n / 2 in each of the half accumulators A and B) over the active list d_list_in: the half-buffer error of
+// every active pixel into the byte mask d_u (W * rows), its box dilation restricted to the active set into d_keep, the final count n
+// into d_samples for the pixels that leave, and the stable compaction of the pixels that stay into d_list_out; their number is written
+// to *count_out (may be pinned host memory).
+struct AdaptiveCheck {
+    const int64_t* d_a;
+    const int64_t* d_b;
+    const uint32_t* d_list_in;
+    uint32_t n_active;
+    uint32_t* d_list_out;
+    uint32_t* count_out;
+    uint8_t* d_u;
+    uint8_t* d_keep;
+    int32_t* d_samples;
+    void* d_temp;        // CUB temp storage of adaptive_select_temp_bytes(n_active or more) bytes
+    size_t temp_bytes;
+    int32_t W, rows, n, radius;
+    double threshold;
+};
+cudaError_t launch_adaptive_iota(uint32_t* d_list, uint32_t n, cudaStream_t stream); // d_list[i] = i
+size_t adaptive_select_temp_bytes(uint32_t max_items);
+cudaError_t launch_adaptive_check(const AdaptiveCheck& c, cudaStream_t stream);
+cudaError_t launch_adaptive_fill(const uint32_t* d_list, uint32_t n_active, int32_t n, int32_t* d_samples, cudaStream_t stream); // samples[list[q]] = n
+// accum_out = A + B, Screen bytes resolved with each pixel's own sample count (0 samples: black)
+cudaError_t launch_resolve_adaptive(const int64_t* d_a, const int64_t* d_b, const int32_t* d_samples, int64_t* d_accum_out, uint8_t* d_screen_u8,
+                                    int32_t W, int32_t H, cudaStream_t stream);
 
 // world.hit for n rays (device pointers)
 cudaError_t launch_trace_batch(const DeviceScene& scene, const rt_ray* d_rays, int64_t n, double t_min, double t_max, int32_t flags, uint64_t seed,

@@ -118,6 +118,33 @@ struct RenderBuffers {
     }
 };
 
+// Working set of rt_render_adaptive, kept between calls like RenderBuffers: the half accumulators A and B, the active pixel list and
+// the next one, per-pixel sample counts, the convergence mask, the compaction flags and CUB's temp storage; the pinned count word the
+// host reads once per check point.
+struct AdaptiveBuffers {
+    int64_t* d_a = nullptr;
+    int64_t* d_b = nullptr;
+    uint32_t* d_list[2] = {nullptr, nullptr};
+    int32_t* d_samples = nullptr;
+    uint8_t* d_u = nullptr;
+    uint8_t* d_keep = nullptr;
+    void* d_temp = nullptr;
+    size_t temp_bytes = 0;
+    uint32_t* h_count = nullptr; // pinned
+    size_t cap = 0;              // pixels (W * H)
+    void release() {
+        if (d_a) cudaFree(d_a);
+        if (d_b) cudaFree(d_b);
+        for (uint32_t*& l : d_list) { if (l) cudaFree(l); l = nullptr; }
+        if (d_samples) cudaFree(d_samples);
+        if (d_u) cudaFree(d_u);
+        if (d_keep) cudaFree(d_keep);
+        if (d_temp) cudaFree(d_temp);
+        if (h_count) cudaFreeHost(h_count);
+        d_a = d_b = nullptr; d_samples = nullptr; d_u = d_keep = nullptr; d_temp = nullptr; temp_bytes = 0; h_count = nullptr; cap = 0;
+    }
+};
+
 // The committed scene on one more GPU (rt_render_multi): same flattened bytes, pointers re-based into this GPU's arena.
 struct Replica {
     int device = -1;
@@ -165,11 +192,13 @@ struct rt_scene {
     RenderTuning tuning;
     Workspace* workspace = nullptr;
     RenderBuffers out;
+    AdaptiveBuffers adaptive;
     std::vector<Replica> replicas; // GPUs 1 .. n-1 of rt_render_multi (GPU 0 is `dev`)
     std::shared_ptr<void> debug_flat; // rt_debug_host_scene: the host-flattened arrays handed to the caller
     ~rt_scene() {
         for (Replica& r : replicas) r.release();
         out.release();
+        adaptive.release();
         dev.release();
         free_workspace(workspace);
     }
@@ -1425,6 +1454,122 @@ int32_t rt_render(rt_scene* s, const rt_render_config* cfg, double* out_screen, 
     return RT_OK;
 }
 
+// ---- adaptive sampling (include/rtb200.h rt_render_adaptive; the numpy mirror is ray_tracing_series_rust_b200/adaptive.py)
+namespace {
+
+int32_t ensure_adaptive_buffers(rt_scene* s, size_t npix) {
+    AdaptiveBuffers& b = s->adaptive;
+    if (npix <= b.cap) return RT_OK;
+    b.release();
+    cudaError_t e;
+    const size_t temp = adaptive_select_temp_bytes((uint32_t)npix);
+    if ((e = cudaMalloc(&b.d_a, npix * 3 * sizeof(int64_t))) != cudaSuccess || (e = cudaMalloc(&b.d_b, npix * 3 * sizeof(int64_t))) != cudaSuccess ||
+        (e = cudaMalloc(&b.d_list[0], npix * sizeof(uint32_t))) != cudaSuccess || (e = cudaMalloc(&b.d_list[1], npix * sizeof(uint32_t))) != cudaSuccess ||
+        (e = cudaMalloc(&b.d_samples, npix * sizeof(int32_t))) != cudaSuccess || (e = cudaMalloc(&b.d_u, npix)) != cudaSuccess ||
+        (e = cudaMalloc(&b.d_keep, npix)) != cudaSuccess || (e = cudaMalloc(&b.d_temp, std::max<size_t>(temp, 1))) != cudaSuccess ||
+        (e = cudaMallocHost(&b.h_count, sizeof(uint32_t))) != cudaSuccess) {
+        b.release();
+        return fail_cuda(e, "adaptive buffers");
+    }
+    b.temp_bytes = temp;
+    b.cap = npix;
+    return RT_OK;
+}
+
+// Counters of several renders into one rt_stats.  concurrent: the renders ran at the same time (rt_render_multi's shards), so
+// iterations and device times are those of the slowest; otherwise (rt_render_adaptive's rounds, one after the other) they add up.
+void add_stats(rt_stats& sum, const rt_stats& r, bool concurrent) {
+    sum.paths += r.paths;
+    sum.segments += r.segments;
+    sum.box_tests += r.box_tests;
+    for (int i = 0; i < 8; ++i) sum.prim_tests[i] += r.prim_tests[i];
+    for (int i = 0; i < 5; ++i) sum.scatters[i] += r.scatters[i];
+    sum.medium_queries += r.medium_queries;
+    sum.kernel_launches += r.kernel_launches;
+    if (concurrent) {
+        sum.iterations = std::max(sum.iterations, r.iterations);
+        sum.ms_device = std::max(sum.ms_device, r.ms_device);
+        sum.ms_extend = std::max(sum.ms_extend, r.ms_extend);
+    } else {
+        sum.iterations += r.iterations;
+        sum.ms_device += r.ms_device;
+        sum.ms_extend += r.ms_extend;
+    }
+}
+
+} // namespace
+
+int32_t rt_render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac, double* out_screen, int64_t* out_accum,
+                           int32_t* out_samples, rt_stats* stats) {
+    CHECK_SCENE(s);
+    if (!cfg) return fail(RT_ERR_INVALID, "null config");
+    // argument checks first: they need no committed scene
+    if (!ac) return fail(RT_ERR_INVALID, "null adaptive config");
+    if (ac->step < 1) return fail(RT_ERR_INVALID, "adaptive step < 1");
+    if (!(ac->threshold >= 0.0) || !std::isfinite(ac->threshold)) return fail(RT_ERR_INVALID, "adaptive threshold must be finite and >= 0");
+    if (ac->radius < 0 || ac->radius > 8) return fail(RT_ERR_INVALID, "adaptive radius outside 0..8");
+    if (ac->min_samples < 0 || ac->min_samples > cfg->samples_per_pixel) return fail(RT_ERR_INVALID, "adaptive min_samples outside 0..samples_per_pixel");
+    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
+        return fail(RT_ERR_INVALID, "rt_render_adaptive takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
+    if (cfg->sample_begin != 0 || (cfg->sample_end != 0 && cfg->sample_end != cfg->samples_per_pixel))
+        return fail(RT_ERR_INVALID, "rt_render_adaptive renders every sample range itself: sample_begin / sample_end must cover [0, samples_per_pixel)");
+    RenderJob job;
+    int32_t rc = make_job(s, cfg, job);
+    if (rc != RT_OK) return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    DeviceGuard guard(s->dev.device);
+    const size_t npix = (size_t)job.width * job.height, n = npix * 3;
+    if ((rc = ensure_out_buffers(s, n)) != RT_OK) return rc;
+    if ((rc = ensure_adaptive_buffers(s, npix)) != RT_OK) return rc;
+    RenderBuffers& o = s->out;
+    AdaptiveBuffers& b = s->adaptive;
+    const RenderTuning tune = tuning_for(s, cfg);
+    const int32_t max = job.spp_total, step = ac->step;
+    const uint32_t rendered = (uint32_t)job.width * (uint32_t)job.rows;
+    cudaError_t e;
+    if ((e = cudaMemsetAsync(b.d_a, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess || (e = cudaMemsetAsync(b.d_b, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess ||
+        (e = cudaMemsetAsync(b.d_samples, 0, npix * sizeof(int32_t), o.stream)) != cudaSuccess || (e = launch_adaptive_iota(b.d_list[0], rendered, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "adaptive set-up");
+    rt_stats sum;
+    std::memset(&sum, 0, sizeof sum);
+    uint32_t n_active = rendered;
+    int cur = 0;
+    for (int64_t k = 0; n_active > 0 && k * step < max; ++k) {
+        const int32_t s0 = (int32_t)(k * step), s1 = (int32_t)std::min<int64_t>((k + 1) * step, max);
+        RenderJob rj = job;
+        rj.sample_begin = s0; rj.sample_end = s1;
+        rj.d_pixels = b.d_list[cur]; rj.n_pixels = n_active;
+        rt_stats rs;
+        std::memset(&rs, 0, sizeof rs);
+        if ((e = launch_render(s->dev.scene, rj, tune, (k & 1) ? b.d_b : b.d_a, o.stream, &rs, &s->workspace)) != cudaSuccess) return fail_cuda(e, "adaptive render round");
+        add_stats(sum, rs, false);
+        if (!(k & 1) || s1 < ac->min_samples || s1 >= max) continue;
+        AdaptiveCheck c;
+        c.d_a = b.d_a; c.d_b = b.d_b;
+        c.d_list_in = b.d_list[cur]; c.n_active = n_active; c.d_list_out = b.d_list[cur ^ 1]; c.count_out = b.h_count;
+        c.d_u = b.d_u; c.d_keep = b.d_keep; c.d_samples = b.d_samples;
+        c.d_temp = b.d_temp; c.temp_bytes = b.temp_bytes;
+        c.W = job.width; c.rows = job.rows; c.n = s1; c.radius = ac->radius; c.threshold = ac->threshold;
+        if ((e = launch_adaptive_check(c, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive check");
+        if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive check sync");
+        n_active = *b.h_count;
+        cur ^= 1;
+    }
+    if ((e = launch_adaptive_fill(b.d_list[cur], n_active, max, b.d_samples, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive counts");
+    if ((e = launch_resolve_adaptive(b.d_a, b.d_b, b.d_samples, o.d_accum, o.d_u8, job.width, job.height, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive resolve");
+    if (out_screen && (e = cudaMemcpyAsync(o.h_u8, o.d_u8, n, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "screen copy");
+    if (out_accum && (e = cudaMemcpyAsync(out_accum, o.d_accum, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "accum copy");
+    if (out_samples && (e = cudaMemcpyAsync(out_samples, b.d_samples, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "samples copy");
+    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive sync");
+    if (out_screen) widen_screen(o.h_u8, out_screen, n);
+    if (stats) {
+        *stats = sum;
+        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    return RT_OK;
+}
+
 // ---- multi-GPU inside the library (SURVEY.md 8(b) n_gpus / shard_mode, 8(e)): one process, N devices
 namespace {
 
@@ -1581,16 +1726,7 @@ int32_t rt_render_multi(rt_scene* s, const rt_render_config* cfg, int32_t n_gpus
     if ((rc = gather_and_copy_out(s, sh, job, out_screen, out_accum)) != RT_OK) return rc;
     if (stats) {
         *stats = st[0];
-        for (int g = 1; g < n_gpus; ++g) {
-            const rt_stats& a = st[(size_t)g];
-            stats->paths += a.paths; stats->segments += a.segments; stats->box_tests += a.box_tests; stats->medium_queries += a.medium_queries;
-            for (int k = 0; k < 8; ++k) stats->prim_tests[k] += a.prim_tests[k];
-            for (int k = 0; k < 5; ++k) stats->scatters[k] += a.scatters[k];
-            stats->iterations = std::max(stats->iterations, a.iterations);
-            stats->kernel_launches += a.kernel_launches;
-            stats->ms_device = std::max(stats->ms_device, a.ms_device); // the slowest shard
-            stats->ms_extend = std::max(stats->ms_extend, a.ms_extend);
-        }
+        for (int g = 1; g < n_gpus; ++g) add_stats(*stats, st[(size_t)g], true); // ms_device: the slowest shard
         stats->kernel_launches += 1; // k_reduce_resolve
         stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     }
