@@ -526,37 +526,64 @@ __global__ void __launch_bounds__(256, RT_SHADE_MIN_BLOCKS) k_shade_all(const __
 // instead of at the ~10 lanes that happen to have ended in this one.  Measured: book-1 final 70.3 -> 68.2 ms (profiles/r2_57_ab_cam_batch.txt);
 // on the sibling-pair kernels of the moving / gravity sphere scenes +-0 / -2.2 % (their walks miss the 9 KB per CTA that the buffer
 // takes from L1), on the same scenes' 4-wide kernels +5.4 % / +0.2 % (r2_67): the three sphere kernels on the 4-wide tree use it
-// (RT_CAM_BATCH = 0: none does).
+// (RT_CAM_BATCH = 0: none does).  The buffer (8.6 KB per CTA) also holds the warps' refill state.
 template <bool ON> struct CamBufferT {
     double v[4][7][32]; // [warp][o.x o.y o.z d.x d.y d.z time][entry]
-    unsigned long long path_id[4][32];
-    uint32_t pixel[4][32], draw[4][32];
+    uint32_t sample[4][32], pixel[4][32], draw[4][32];
+    // The warp-uniform refill state: read and written once per refill, so it lives here rather than in 7 registers of every lane for
+    // the whole kernel (part of what fits the kernel into 80 registers, 6 CTAs/SM)
+    unsigned long long chunk_next[4], chunk_end[4];
+    uint32_t head[4], count[4], gen_done[4]; // gen_done: the path indices have run out
+    uint32_t dry[4];                         // gen_done and the buffer is empty: idle lanes of the warp stay idle
 };
 template <> struct CamBufferT<false> {};
-template <bool MEDIA, int MINB, bool GENERAL_MEDIA, uint32_t PM = RT_PM_ALL, bool XF = true, bool WIDE = false>
+// What a lane keeps of its path besides the ray: read and written in the shading code only, never in the walk.  The camera-batch kernels
+// keep it in shared memory ([thread], 9 words: an odd stride, conflict free), so that it takes no registers while the lane walks the tree.
+struct PathVars {
+    float tr, tg, tb;             // throughput (world.rs:57 `product`)
+    uint32_t pixel, sample, draw; // the path id pixel * spp_total + sample is formed where Philox needs it; Philox draw counter
+    uint32_t segment, segs, pad;  // ray_color iteration; segments this lane has traced (statistics)
+};
+template <bool SMEM> struct PathVarsT {};
+template <> struct PathVarsT<true> { PathVars v[128]; };
+template <bool SMEM> RT_DEV PathVars& path_vars(PathVarsT<SMEM>& sm, PathVars& reg) {
+    if constexpr (SMEM) return sm.v[threadIdx.x];
+    else return reg;
+}
+// FULLTEX = false: the scene has no Noise and no Image texture (DeviceScene::flags bits 3 and 4 clear): the Perlin and texel code and the
+// sphere (u, v) are compiled out.  The Perlin turbulence is the register peak of the kernel (tools/reg_pressure.py: 93 live at 5 CTAs/SM).
+template <bool MEDIA, int MINB, bool GENERAL_MEDIA, uint32_t PM = RT_PM_ALL, bool XF = true, bool WIDE = false, bool FULLTEX = true>
 __global__ void __launch_bounds__(128, MINB) k_mega(const __grid_constant__ DeviceScene S, const __grid_constant__ JobDev J, Queues Q,
                                                       int64_t* __restrict__ accum) {
     const unsigned full = 0xffffffffu;
-    unsigned long long chunk_next = 0, chunk_end = 0; // warp-uniform
+    unsigned long long chunk_next = 0, chunk_end = 0; // warp-uniform (the camera-batch kernels keep theirs in CamBufferT)
     Ray r;
     r.o = mk3(0, 0, 0); r.d = mk3(0, 0, 1); r.time = 0.0;
-    float tr = 0.f, tg = 0.f, tb = 0.f;
-    uint32_t pixel = 0, draw = 0, segment = 0;
-    uint64_t path_id = 0;
     bool alive = false, exhausted = false;
-    uint32_t my_segments = 0;
     constexpr bool CAMB = RT_CAM_BATCH && WIDE && (PM == 0x1u || PM == 0x3u || PM == 0x5u);
     __shared__ CamBufferT<CAMB> cam;
+    __shared__ PathVarsT<CAMB> pv_smem;
+    PathVars pv_reg;
+    PathVars& pv = path_vars<CAMB>(pv_smem, pv_reg);
+    pv.tr = pv.tg = pv.tb = 0.f;
+    pv.pixel = 0; pv.sample = 0; pv.draw = 0; pv.segment = 0; pv.segs = 0;
     const uint32_t wid = threadIdx.x >> 5, ln = lane_id();
-    uint32_t buf_head = 0, buf_count = 0; // warp-uniform
-    bool gen_done = false;                // warp-uniform: the path indices have run out
+    if constexpr (CAMB) {
+        if (ln == 0) { cam.chunk_next[wid] = 0; cam.chunk_end[wid] = 0; cam.head[wid] = 0; cam.count[wid] = 0; cam.gen_done[wid] = 0; cam.dry[wid] = 0; }
+        __syncwarp();
+    }
     for (;;) {
         // ---- refill idle lanes
-        const unsigned need = __ballot_sync(full, !alive && !exhausted);
+        bool idle = !alive; // and not out of work: `exhausted`, which the camera-batch kernels keep per warp (dry) instead of per lane
+        if constexpr (CAMB) idle = idle && cam.dry[wid] == 0u;
+        else idle = idle && !exhausted;
+        const unsigned need = __ballot_sync(full, idle);
         if constexpr (CAMB) {
           if (need) {
+            uint32_t buf_head = cam.head[wid], buf_count = cam.count[wid];
+            bool gen_done = cam.gen_done[wid] != 0;
             uint32_t rank = __popc(need & ((1u << ln) - 1u));
-            bool want = !alive && !exhausted;
+            bool want = idle;
             for (int round = 0; round < 2; ++round) { // what the buffer holds first; then, if lanes are left over, 32 new rays and the rest
                 const uint32_t want_n = __popc(__ballot_sync(full, want));
                 const uint32_t served = want_n < buf_count ? want_n : buf_count;
@@ -565,9 +592,9 @@ __global__ void __launch_bounds__(128, MINB) k_mega(const __grid_constant__ Devi
                     r.o = mk3(cam.v[wid][0][e], cam.v[wid][1][e], cam.v[wid][2][e]);
                     r.d = mk3(cam.v[wid][3][e], cam.v[wid][4][e], cam.v[wid][5][e]);
                     r.time = cam.v[wid][6][e];
-                    path_id = cam.path_id[wid][e]; pixel = cam.pixel[wid][e]; draw = cam.draw[wid][e];
-                    tr = tg = tb = 1.f;
-                    segment = 0;
+                    pv.sample = cam.sample[wid][e]; pv.pixel = cam.pixel[wid][e]; pv.draw = cam.draw[wid][e];
+                    pv.tr = pv.tg = pv.tb = 1.f;
+                    pv.segment = 0;
                     alive = true;
                     want = false;
                 } else if (want) {
@@ -575,37 +602,46 @@ __global__ void __launch_bounds__(128, MINB) k_mega(const __grid_constant__ Devi
                 }
                 buf_head += served; buf_count -= served;
                 if (served == want_n) break;
-                if (round == 1 || gen_done) { if (want) exhausted = true; break; }
+                if (round == 1 || gen_done) break; // lanes still wanting are out of work: the buffer is empty and gen_done is set
                 // the buffer is empty: the whole warp generates the next 32 camera rays
                 __syncwarp();
-                if (chunk_next == chunk_end) {
+                unsigned long long c_next = cam.chunk_next[wid], c_end = cam.chunk_end[wid];
+                if (c_next == c_end) {
                     unsigned long long base = 0;
                     uint32_t got = 0;
                     if (ln == 0) base = claim_chunk(J, Q, got);
                     base = __shfl_sync(full, base, 0);
                     got = __shfl_sync(full, got, 0);
-                    chunk_next = base; chunk_end = base + got;
+                    c_next = base; c_end = base + got;
                 }
-                const unsigned long long L = chunk_next + ln;
-                chunk_next += 32;
+                const unsigned long long L = c_next + ln;
                 const bool valid = L < J.total_paths;
                 if (valid) {
                     uint32_t s_local, pix, d0;
                     split_path_index(L + J.path_base, J.npix_rendered, s_local, pix);
                     pix = shard_pixel(J, pix);
                     const int32_t j = (int32_t)(pix / (uint32_t)J.W), ii = (int32_t)(pix - (uint32_t)j * (uint32_t)J.W);
-                    const uint64_t pid = (uint64_t)pix * (uint64_t)J.spp_total + (uint64_t)(J.sample_begin + (int32_t)s_local);
+                    const uint32_t smp = (uint32_t)(J.sample_begin + (int32_t)s_local);
+                    const uint64_t pid = (uint64_t)pix * (uint64_t)J.spp_total + (uint64_t)smp;
                     const Ray cr = camera_first_ray<PathRngOol>(S.cam, ii, j, J.W, J.H, J.seed, pid, d0); // world.rs:1212-1214
                     cam.v[wid][0][ln] = cr.o.x; cam.v[wid][1][ln] = cr.o.y; cam.v[wid][2][ln] = cr.o.z;
                     cam.v[wid][3][ln] = cr.d.x; cam.v[wid][4][ln] = cr.d.y; cam.v[wid][5][ln] = cr.d.z;
                     cam.v[wid][6][ln] = cr.time;
-                    cam.path_id[wid][ln] = pid; cam.pixel[wid][ln] = pix; cam.draw[wid][ln] = d0;
+                    cam.sample[wid][ln] = smp; cam.pixel[wid][ln] = pix; cam.draw[wid][ln] = d0;
                 }
                 buf_head = 0;
                 buf_count = __popc(__ballot_sync(full, valid)); // valid lanes are a prefix: L grows with the lane
                 if (buf_count < 32u) gen_done = true;
                 __syncwarp();
+                if (ln == 0) { cam.chunk_next[wid] = c_next + 32; cam.chunk_end[wid] = c_end; }
+                __syncwarp();
             }
+            __syncwarp();
+            if (ln == 0) {
+                cam.head[wid] = buf_head; cam.count[wid] = buf_count; cam.gen_done[wid] = gen_done ? 1u : 0u;
+                cam.dry[wid] = (gen_done && buf_count == 0u) ? 1u : 0u;
+            }
+            __syncwarp();
           }
         } else if (need) {
             const uint32_t n_need = __popc(need);
@@ -625,13 +661,13 @@ __global__ void __launch_bounds__(128, MINB) k_mega(const __grid_constant__ Devi
                     exhausted = true;
                 } else {
                     uint32_t s_local;
-                    split_path_index(L + J.path_base, J.npix_rendered, s_local, pixel);
-                    pixel = shard_pixel(J, pixel);
-                    const int32_t j = (int32_t)(pixel / (uint32_t)J.W), ii = (int32_t)(pixel - (uint32_t)j * (uint32_t)J.W);
-                    path_id = (uint64_t)pixel * (uint64_t)J.spp_total + (uint64_t)(J.sample_begin + (int32_t)s_local);
-                    r = camera_first_ray<PathRngOol>(S.cam, ii, j, J.W, J.H, J.seed, path_id, draw); // world.rs:1212-1214
-                    tr = tg = tb = 1.f;
-                    segment = 0;
+                    split_path_index(L + J.path_base, J.npix_rendered, s_local, pv.pixel);
+                    pv.pixel = shard_pixel(J, pv.pixel);
+                    const int32_t j = (int32_t)(pv.pixel / (uint32_t)J.W), ii = (int32_t)(pv.pixel - (uint32_t)j * (uint32_t)J.W);
+                    pv.sample = (uint32_t)(J.sample_begin + (int32_t)s_local);
+                    r = camera_first_ray<PathRngOol>(S.cam, ii, j, J.W, J.H, J.seed, (uint64_t)pv.pixel * (uint64_t)J.spp_total + (uint64_t)pv.sample, pv.draw); // world.rs:1212-1214
+                    pv.tr = pv.tg = pv.tb = 1.f;
+                    pv.segment = 0;
                     alive = true;
                 }
             }
@@ -651,48 +687,49 @@ __global__ void __launch_bounds__(128, MINB) k_mega(const __grid_constant__ Devi
             int sp = 0;
             trace_wide<PM, false>(S, r, 0.001, best, cur, sp, wstack, 0u);
             hit = best.type != RT_NONE;
-            if (hit) h = finalize_hit<2, PM, false>(S, r, best);
+            if (hit) h = finalize_hit<FULLTEX ? 2 : 0, PM, false>(S, r, best);
         } else {
-            hit = world_hit<false, 2, MEDIA, GENERAL_MEDIA, PM, XF>(S, r, 0.001, RT_INF, true, J.seed, path_id, segment, h, nullptr);
+            hit = world_hit<false, 2, MEDIA, GENERAL_MEDIA, PM, XF>(S, r, 0.001, RT_INF, true, J.seed, (uint64_t)pv.pixel * (uint64_t)J.spp_total + (uint64_t)pv.sample,
+                                                                    pv.segment, h, nullptr);
         }
-        ++my_segments;
+        ++pv.segs;
         F3 contrib = mkf3(0.f, 0.f, 0.f);
         bool ended = true;
         if (!hit) {
             const F3 bg = miss_color(S, r.d);
-            contrib = mkf3(tr * bg.x, tg * bg.y, tb * bg.z);
+            contrib = mkf3(pv.tr * bg.x, pv.tg * bg.y, pv.tb * bg.z);
         } else {
             const DMaterial m = S.materials[h.mat];
             if (m.type == MAT_LIGHT) {
-                const F3 e = tex_value(S, m.tex, h.u, h.v, h.p);
-                contrib = mkf3(tr * e.x, tg * e.y, tb * e.z);
+                const F3 e = tex_value<FULLTEX>(S, m.tex, h.u, h.v, h.p);
+                contrib = mkf3(pv.tr * e.x, pv.tg * e.y, pv.tb * e.z);
             } else {
                 PathRngOolBegun g;
-                g.init(J.seed, path_id, draw);
+                g.init(J.seed, (uint64_t)pv.pixel * (uint64_t)J.spp_total + (uint64_t)pv.sample, pv.draw);
                 g.open_event(); // Material::scatter starts on a block boundary: the first block for every scattering lane at once
                 D3 dir = mk3(0, 0, 0), rs = mk3(0, 0, 0);
                 F3 att = mkf3(0.f, 0.f, 0.f);
                 bool scattered;
                 if (m.type != MAT_DIELECTRIC) rs = random_in_unit_sphere(g); // one rejection loop for Lambertian, Metal and Isotropic lanes
-                if (m.type == MAT_LAMBERTIAN) scattered = lambertian_finish(S, m, h.p, h.n, h.u, h.v, rs, dir, att);
+                if (m.type == MAT_LAMBERTIAN) scattered = lambertian_finish<FULLTEX>(S, m, h.p, h.n, h.u, h.v, rs, dir, att);
                 else if (m.type == MAT_METAL) scattered = metal_finish(m, r.d, h.n, rs, dir, att);
                 else if (m.type == MAT_DIELECTRIC) scattered = scatter_dielectric(m, r.d, h.n, h.front, g, dir, att);
-                else scattered = isotropic_finish(S, m, h.p, h.u, h.v, rs, dir, att);
-                if (scattered && (int32_t)(segment + 1) < J.max_depth) {
-                    tr *= att.x; tg *= att.y; tb *= att.z;
+                else scattered = isotropic_finish<FULLTEX>(S, m, h.p, h.u, h.v, rs, dir, att);
+                if (scattered && (int32_t)(pv.segment + 1) < J.max_depth) {
+                    pv.tr *= att.x; pv.tg *= att.y; pv.tb *= att.z;
                     r.o = h.p; r.d = dir;
-                    draw = g.draw;
-                    ++segment;
+                    pv.draw = g.draw;
+                    ++pv.segment;
                     ended = false;
                 }
             }
         }
         if (ended) {
-            accumulate(accum, pixel, contrib.x, contrib.y, contrib.z);
+            accumulate(accum, pv.pixel, contrib.x, contrib.y, contrib.z);
             alive = false;
         }
     }
-    uint32_t segs = my_segments;
+    uint32_t segs = pv.segs;
     for (int o = 16; o > 0; o >>= 1) segs += __shfl_xor_sync(full, segs, o);
     if (lane_id() == 0 && segs) atomicAdd(&Q.stats[0], (unsigned long long)segs);
 }
@@ -1395,6 +1432,20 @@ static void launch_pool(cudaStream_t st, const DeviceScene& scene, const JobDev&
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); // per device: set on every launch (microseconds)
     kern<<<148 * MINB, 128, smem, st>>>(scene, J, Q, d_accum);
 }
+// Resident CTAs per SM of the 4-wide sphere kernels (spheres, + moving spheres, + gravity spheres; no Noise / Image texture): the kernel is
+// compiled for it (__launch_bounds__) and launched with 148 x that many CTAs.  6 needs <= 80 registers, 7 <= 72; see
+// build/kernels.ptxas.log and tools/reg_pressure.py for what ptxas made of it.  Measured against 5 (profiles/r3_01_ab_occ_sph.txt):
+// book-1 final 68.06 -> 64.56 ms (80 registers, no spills), book-1 as shipped 48.98 -> 47.66 ms (80 registers, 52 B of spill stores:
+// hit point and normal around the scatter), bouncing-spheres frame 64.34 -> 59.37 ms (no spills).  At 7 all three spill.
+#ifndef RT_MEGA_OCC_SPH
+#define RT_MEGA_OCC_SPH 6
+#endif
+template <uint32_t PM>
+static void launch_mega_wide_sph(cudaStream_t st, const DeviceScene& scene, const JobDev& J, const Queues& Q, int64_t* d_accum) {
+    constexpr int OCC = RT_MEGA_OCC_SPH;
+    if (scene.flags & 24u) k_mega<false, 5, false, PM, false, true, true><<<148 * 5, 128, 0, st>>>(scene, J, Q, d_accum); // Perlin / image textures
+    else k_mega<false, OCC, false, PM, false, true, false><<<148 * OCC, 128, 0, st>>>(scene, J, Q, d_accum);
+}
 cudaError_t launch_render(const DeviceScene& scene, const RenderJob& job, const RenderTuning& tune, int64_t* d_accum, cudaStream_t stream,
                           rt_stats* stats, Workspace** wsp) {
     cudaError_t err = cudaSuccess;
@@ -1486,7 +1537,8 @@ cudaError_t launch_render(const DeviceScene& scene, const RenderJob& job, const 
             k_mega_init<<<1, 32, 0, stream>>>(Q);
             // Variant choice (every step A/B-measured on B200, DESIGN.md section 5): compile-time primitive mask when the scene
             // holds only spheres / spheres + moving spheres / rects + triangles; wrapper-free (XF = false) variants at 5 CTAs/SM
-            // (96 registers, no spills), everything else at 4 (128 registers); media: 4, or 3 with the general two-traversal path.
+            // (96 registers), the 4-wide sphere kernels at RT_MEGA_OCC_SPH (80 registers) unless the scene has Noise / Image textures,
+            // everything else at 4 (128 registers); media: 4, or 3 with the general two-traversal path.
             const uint32_t pm = !tune.prim_specialise ? RT_PM_ALL
                                 : (scene.prim_mask == 0x1u ? 0x1u : ((scene.prim_mask & ~0x3u) == 0 ? 0x3u : ((scene.prim_mask & ~0x5u) == 0 ? 0x5u : ((scene.prim_mask & ~0x28u) == 0 ? 0x28u : RT_PM_ALL))));
             // Path indices are claimed per warp in chunks of consecutive indices (neighbouring pixels of one sample).  512 is best for
@@ -1520,9 +1572,9 @@ cudaError_t launch_render(const DeviceScene& scene, const RenderJob& job, const 
                     k_mega_r<7, 0x28u, true><<<148 * 7, 128, 0, stream>>>(scene, J, Q, d_accum);
                 } else k_mega_r<7, 0x28u><<<148 * 7, 128, 0, stream>>>(scene, J, Q, d_accum);
             } else if (wrapper_free && scene.nodes4 && tune.bvh_wide != 0 && scene.n_main_instances == 1 && (pm == 0x1u || pm == 0x3u || pm == 0x5u || pm == 0x28u)) {
-                if (pm == 0x1u) k_mega<false, 5, false, 0x1u, false, true><<<148 * 5, 128, 0, stream>>>(scene, J, Q, d_accum);
-                else if (pm == 0x3u) k_mega<false, 5, false, 0x3u, false, true><<<148 * 5, 128, 0, stream>>>(scene, J, Q, d_accum); // motion form (mnodes4), forced only
-                else if (pm == 0x5u) k_mega<false, 5, false, 0x5u, false, true><<<148 * 5, 128, 0, stream>>>(scene, J, Q, d_accum);
+                if (pm == 0x1u) launch_mega_wide_sph<0x1u>(stream, scene, J, Q, d_accum);
+                else if (pm == 0x3u) launch_mega_wide_sph<0x3u>(stream, scene, J, Q, d_accum); // motion form (mnodes4)
+                else if (pm == 0x5u) launch_mega_wide_sph<0x5u>(stream, scene, J, Q, d_accum);
                 else k_mega<false, 5, false, 0x28u, false, true><<<148 * 5, 128, 0, stream>>>(scene, J, Q, d_accum);
             } else if (wrapper_free && pm != RT_PM_ALL) {
                 if (pm == 0x1u) k_mega<false, 5, false, 0x1u, false><<<148 * 5, 128, 0, stream>>>(scene, J, Q, d_accum);       // book-1 final

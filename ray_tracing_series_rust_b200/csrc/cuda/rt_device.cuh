@@ -641,6 +641,34 @@ RT_DEV unsigned long long wide_key_nf(float nx, float fx, float ny, float fy, fl
     if (!(tn <= tf)) return ~0ull;
     return ((unsigned long long)(__float_as_uint(tn) & 0x7fffffffu) << 32) | (unsigned long long)__float_as_uint(ref);
 }
+RT_DEV float4 wide_lerp(float4 v, float4 d, float ms) { return make_float4(fmaf(d.x, ms, v.x), fmaf(d.y, ms, v.y), fmaf(d.z, ms, v.z), fmaf(d.w, ms, v.w)); }
+// The near and far row of one axis (q = the node's row pair of that axis, sg = the ray's byte offset of its near row); `motion`: the
+// rows of the motion nodes (DeviceScene::mnodes4) interpolated to the ray's shutter position ms
+RT_DEV void wide_rows(const float4* q, uint32_t sg, bool motion, float ms, float4& n, float4& fr) {
+    const float4* qn = wide_row(q, sg);
+    const float4* qf = wide_row(q, sg ^ 16u);
+    n = __ldg(qn); fr = __ldg(qf);
+    if (motion) { n = wide_lerp(n, __ldg(qn + 8), ms); fr = wide_lerp(fr, __ldg(qf + 8), ms); }
+}
+// The signed-row key of the four children of a node, an axis at a time: fmaxf / fminf return one of their operands (the non-NaN one),
+// so the running max(max(max(x, t_min), y), z) is the value of max(max(x, y), max(z, t_min)) (up to the sign of a zero, which the key
+// masks off and tn <= tf does not see): the same keys, bit for bit
+RT_DEV void wide_fold_x(const float4& n, const float4& fr, const RayF& f, float t_min, float t_max, float4& tn, float4& tf) {
+    tn.x = fmaxf(fmaf(n.x, f.idx, -f.oodx), t_min); tf.x = fminf(fmaf(fr.x, f.idx, -f.oodx), t_max);
+    tn.y = fmaxf(fmaf(n.y, f.idx, -f.oodx), t_min); tf.y = fminf(fmaf(fr.y, f.idx, -f.oodx), t_max);
+    tn.z = fmaxf(fmaf(n.z, f.idx, -f.oodx), t_min); tf.z = fminf(fmaf(fr.z, f.idx, -f.oodx), t_max);
+    tn.w = fmaxf(fmaf(n.w, f.idx, -f.oodx), t_min); tf.w = fminf(fmaf(fr.w, f.idx, -f.oodx), t_max);
+}
+RT_DEV void wide_fold(const float4& n, const float4& fr, float id, float ood, float4& tn, float4& tf) {
+    tn.x = fmaxf(tn.x, fmaf(n.x, id, -ood)); tf.x = fminf(tf.x, fmaf(fr.x, id, -ood));
+    tn.y = fmaxf(tn.y, fmaf(n.y, id, -ood)); tf.y = fminf(tf.y, fmaf(fr.y, id, -ood));
+    tn.z = fmaxf(tn.z, fmaf(n.z, id, -ood)); tf.z = fminf(tf.z, fmaf(fr.z, id, -ood));
+    tn.w = fmaxf(tn.w, fmaf(n.w, id, -ood)); tf.w = fminf(tf.w, fmaf(fr.w, id, -ood));
+}
+RT_DEV unsigned long long wide_key_tn(float tn, float tf, float ref) {
+    if (!(tn <= tf)) return ~0ull;
+    return ((unsigned long long)(__float_as_uint(tn) & 0x7fffffffu) << 32) | (unsigned long long)__float_as_uint(ref);
+}
 #ifndef RT_WIDE_CE32
 #define RT_WIDE_CE32 1
 #endif
@@ -701,46 +729,69 @@ RT_DEV void walk_wide(const DeviceScene& S, const Ray& r, const RayF& f, const R
 #define RT_INNER_MEDIA 1 // the media wavefront kernels' masks (rects + boxes, + spheres + moving spheres): 1 / 2 / unbounded measured, 1 is best
 #endif
         constexpr int INNER = RT_PM_HAS(PM, PRIM_TRI) ? RT_INNER_TRI : ((PM == 0x18u || PM == 0x1bu) ? RT_INNER_MEDIA : RT_INNER_SPH);
+        // The sphere kernels (k_mega at 80 registers) load and fold the node one axis at a time: fewer rows live at once.  The triangle
+        // and media kernels keep all seven rows in flight (the fold measured -2.9 % on the 871 200-triangle mesh, -0.7 % on book-2 final)
+        constexpr bool WIDE_FOLD = PM == 0x1u || PM == 0x3u || PM == 0x5u;
 #pragma unroll 1
         for (int inner = 0; inner < INNER && cur != DONE && !(cur & RT_LEAF_FLAG); ++inner) {
-            float4 lx, hx, ly, hy, lz, hz, rf;
-            if (MOTION) { // box(t) = box at the shutter's start + s * delta: 256 bytes per node
-                // (signed rows as below: start and end boxes are valid and the interpolation is monotonic, so lo(t) <= hi(t) holds)
-                const float4* __restrict__ q = mnodes4 + 16 * (size_t)cur;
-                const float4* qx = RT_WIDE_SIGNED ? wide_row(q, sgx) : q;
-                const float4* qX = RT_WIDE_SIGNED ? wide_row(q, sgx ^ 16u) : q + 1;
-                const float4* qy = RT_WIDE_SIGNED ? wide_row(q, sgy) + 2 : q + 2;
-                const float4* qY = RT_WIDE_SIGNED ? wide_row(q, sgy ^ 16u) + 2 : q + 3;
-                const float4* qz = RT_WIDE_SIGNED ? wide_row(q, sgz) + 4 : q + 4;
-                const float4* qZ = RT_WIDE_SIGNED ? wide_row(q, sgz ^ 16u) + 4 : q + 5;
-                lx = __ldg(qx); hx = __ldg(qX); ly = __ldg(qy); hy = __ldg(qY); lz = __ldg(qz); hz = __ldg(qZ); rf = __ldg(q + 6);
-                const float4 dlx = __ldg(qx + 8), dhx = __ldg(qX + 8), dly = __ldg(qy + 8), dhy = __ldg(qY + 8), dlz = __ldg(qz + 8), dhz = __ldg(qZ + 8);
-                lx.x = fmaf(dlx.x, ms, lx.x); lx.y = fmaf(dlx.y, ms, lx.y); lx.z = fmaf(dlx.z, ms, lx.z); lx.w = fmaf(dlx.w, ms, lx.w);
-                hx.x = fmaf(dhx.x, ms, hx.x); hx.y = fmaf(dhx.y, ms, hx.y); hx.z = fmaf(dhx.z, ms, hx.z); hx.w = fmaf(dhx.w, ms, hx.w);
-                ly.x = fmaf(dly.x, ms, ly.x); ly.y = fmaf(dly.y, ms, ly.y); ly.z = fmaf(dly.z, ms, ly.z); ly.w = fmaf(dly.w, ms, ly.w);
-                hy.x = fmaf(dhy.x, ms, hy.x); hy.y = fmaf(dhy.y, ms, hy.y); hy.z = fmaf(dhy.z, ms, hy.z); hy.w = fmaf(dhy.w, ms, hy.w);
-                lz.x = fmaf(dlz.x, ms, lz.x); lz.y = fmaf(dlz.y, ms, lz.y); lz.z = fmaf(dlz.z, ms, lz.z); lz.w = fmaf(dlz.w, ms, lz.w);
-                hz.x = fmaf(dhz.x, ms, hz.x); hz.y = fmaf(dhz.y, ms, hz.y); hz.z = fmaf(dhz.z, ms, hz.z); hz.w = fmaf(dhz.w, ms, hz.w);
-            } else if (RT_WIDE_SIGNED) { // rows picked by the ray's direction signs: l* = the planes it enters through, h* = leaves through
-                const float4* __restrict__ q = nodes4 + 8 * (size_t)cur;
-                lx = __ldg(wide_row(q, sgx)); hx = __ldg(wide_row(q, sgx ^ 16u)); ly = __ldg(wide_row(q, sgy) + 2); hy = __ldg(wide_row(q, sgy ^ 16u) + 2);
-                lz = __ldg(wide_row(q, sgz) + 4); hz = __ldg(wide_row(q, sgz ^ 16u) + 4); rf = __ldg(q + 6);
-            } else {
-                const float4* __restrict__ q = nodes4 + 8 * (size_t)cur;
-                lx = __ldg(q); hx = __ldg(q + 1); ly = __ldg(q + 2); hy = __ldg(q + 3); lz = __ldg(q + 4); hz = __ldg(q + 5); rf = __ldg(q + 6);
-            }
-            if (COUNT) cnt->nodes += 4;
             unsigned long long k0, k1, k2, k3;
-            if (RT_WIDE_SIGNED) {
-                k0 = wide_key_nf(lx.x, hx.x, ly.x, hy.x, lz.x, hz.x, rf.x, f, tminf, tmaxf);
-                k1 = wide_key_nf(lx.y, hx.y, ly.y, hy.y, lz.y, hz.y, rf.y, f, tminf, tmaxf);
-                k2 = wide_key_nf(lx.z, hx.z, ly.z, hy.z, lz.z, hz.z, rf.z, f, tminf, tmaxf);
-                k3 = wide_key_nf(lx.w, hx.w, ly.w, hy.w, lz.w, hz.w, rf.w, f, tminf, tmaxf);
+            if constexpr (RT_WIDE_SIGNED && WIDE_FOLD) { // rows picked by the ray's direction signs: near = the planes it enters through, far = leaves through
+                if (COUNT) cnt->nodes += 4;
+                // MOTION: box(t) = box at the shutter's start + s * delta, 256 bytes per node (start and end boxes are valid and the
+                // interpolation is monotonic, so lo(t) <= hi(t) holds and the signed rows stay right)
+                const float4* __restrict__ q = MOTION ? mnodes4 + 16 * (size_t)cur : nodes4 + 8 * (size_t)cur;
+                // one axis at a time, folded into running near / far values: a pair of rows is dead before the next one is needed
+                float4 n, fr, tn, tf;
+                wide_rows(q, sgx, MOTION, ms, n, fr);
+                wide_fold_x(n, fr, f, tminf, tmaxf, tn, tf);
+                wide_rows(q + 2, sgy, MOTION, ms, n, fr);
+                wide_fold(n, fr, f.idy, f.oody, tn, tf);
+                wide_rows(q + 4, sgz, MOTION, ms, n, fr);
+                wide_fold(n, fr, f.idz, f.oodz, tn, tf);
+                const float4 rf = __ldg(q + 6);
+                k0 = wide_key_tn(tn.x, tf.x, rf.x);
+                k1 = wide_key_tn(tn.y, tf.y, rf.y);
+                k2 = wide_key_tn(tn.z, tf.z, rf.z);
+                k3 = wide_key_tn(tn.w, tf.w, rf.w);
             } else {
-                k0 = wide_key(lx.x, hx.x, ly.x, hy.x, lz.x, hz.x, rf.x, f, tminf, tmaxf);
-                k1 = wide_key(lx.y, hx.y, ly.y, hy.y, lz.y, hz.y, rf.y, f, tminf, tmaxf);
-                k2 = wide_key(lx.z, hx.z, ly.z, hy.z, lz.z, hz.z, rf.z, f, tminf, tmaxf);
-                k3 = wide_key(lx.w, hx.w, ly.w, hy.w, lz.w, hz.w, rf.w, f, tminf, tmaxf);
+                float4 lx, hx, ly, hy, lz, hz, rf;
+                if (MOTION) { // box(t) = box at the shutter's start + s * delta: 256 bytes per node
+                    // (signed rows as below: start and end boxes are valid and the interpolation is monotonic, so lo(t) <= hi(t) holds)
+                    const float4* __restrict__ q = mnodes4 + 16 * (size_t)cur;
+                    const float4* qx = RT_WIDE_SIGNED ? wide_row(q, sgx) : q;
+                    const float4* qX = RT_WIDE_SIGNED ? wide_row(q, sgx ^ 16u) : q + 1;
+                    const float4* qy = RT_WIDE_SIGNED ? wide_row(q, sgy) + 2 : q + 2;
+                    const float4* qY = RT_WIDE_SIGNED ? wide_row(q, sgy ^ 16u) + 2 : q + 3;
+                    const float4* qz = RT_WIDE_SIGNED ? wide_row(q, sgz) + 4 : q + 4;
+                    const float4* qZ = RT_WIDE_SIGNED ? wide_row(q, sgz ^ 16u) + 4 : q + 5;
+                    lx = __ldg(qx); hx = __ldg(qX); ly = __ldg(qy); hy = __ldg(qY); lz = __ldg(qz); hz = __ldg(qZ); rf = __ldg(q + 6);
+                    const float4 dlx = __ldg(qx + 8), dhx = __ldg(qX + 8), dly = __ldg(qy + 8), dhy = __ldg(qY + 8), dlz = __ldg(qz + 8), dhz = __ldg(qZ + 8);
+                    lx.x = fmaf(dlx.x, ms, lx.x); lx.y = fmaf(dlx.y, ms, lx.y); lx.z = fmaf(dlx.z, ms, lx.z); lx.w = fmaf(dlx.w, ms, lx.w);
+                    hx.x = fmaf(dhx.x, ms, hx.x); hx.y = fmaf(dhx.y, ms, hx.y); hx.z = fmaf(dhx.z, ms, hx.z); hx.w = fmaf(dhx.w, ms, hx.w);
+                    ly.x = fmaf(dly.x, ms, ly.x); ly.y = fmaf(dly.y, ms, ly.y); ly.z = fmaf(dly.z, ms, ly.z); ly.w = fmaf(dly.w, ms, ly.w);
+                    hy.x = fmaf(dhy.x, ms, hy.x); hy.y = fmaf(dhy.y, ms, hy.y); hy.z = fmaf(dhy.z, ms, hy.z); hy.w = fmaf(dhy.w, ms, hy.w);
+                    lz.x = fmaf(dlz.x, ms, lz.x); lz.y = fmaf(dlz.y, ms, lz.y); lz.z = fmaf(dlz.z, ms, lz.z); lz.w = fmaf(dlz.w, ms, lz.w);
+                    hz.x = fmaf(dhz.x, ms, hz.x); hz.y = fmaf(dhz.y, ms, hz.y); hz.z = fmaf(dhz.z, ms, hz.z); hz.w = fmaf(dhz.w, ms, hz.w);
+                } else if (RT_WIDE_SIGNED) { // rows picked by the ray's direction signs: l* = the planes it enters through, h* = leaves through
+                    const float4* __restrict__ q = nodes4 + 8 * (size_t)cur;
+                    lx = __ldg(wide_row(q, sgx)); hx = __ldg(wide_row(q, sgx ^ 16u)); ly = __ldg(wide_row(q, sgy) + 2); hy = __ldg(wide_row(q, sgy ^ 16u) + 2);
+                    lz = __ldg(wide_row(q, sgz) + 4); hz = __ldg(wide_row(q, sgz ^ 16u) + 4); rf = __ldg(q + 6);
+                } else {
+                    const float4* __restrict__ q = nodes4 + 8 * (size_t)cur;
+                    lx = __ldg(q); hx = __ldg(q + 1); ly = __ldg(q + 2); hy = __ldg(q + 3); lz = __ldg(q + 4); hz = __ldg(q + 5); rf = __ldg(q + 6);
+                }
+                if (COUNT) cnt->nodes += 4;
+                if (RT_WIDE_SIGNED) {
+                    k0 = wide_key_nf(lx.x, hx.x, ly.x, hy.x, lz.x, hz.x, rf.x, f, tminf, tmaxf);
+                    k1 = wide_key_nf(lx.y, hx.y, ly.y, hy.y, lz.y, hz.y, rf.y, f, tminf, tmaxf);
+                    k2 = wide_key_nf(lx.z, hx.z, ly.z, hy.z, lz.z, hz.z, rf.z, f, tminf, tmaxf);
+                    k3 = wide_key_nf(lx.w, hx.w, ly.w, hy.w, lz.w, hz.w, rf.w, f, tminf, tmaxf);
+                } else {
+                    k0 = wide_key(lx.x, hx.x, ly.x, hy.x, lz.x, hz.x, rf.x, f, tminf, tmaxf);
+                    k1 = wide_key(lx.y, hx.y, ly.y, hy.y, lz.y, hz.y, rf.y, f, tminf, tmaxf);
+                    k2 = wide_key(lx.z, hx.z, ly.z, hy.z, lz.z, hz.z, rf.z, f, tminf, tmaxf);
+                    k3 = wide_key(lx.w, hx.w, ly.w, hy.w, lz.w, hz.w, rf.w, f, tminf, tmaxf);
+                }
             }
             // Only the nearest child is found exactly (three compare-exchanges); k1..k3 are pushed as they are.  The full five-exchange
             // sort (far-to-near pushes) measured 2.7 % slower on book-1 final and 3 % on the 871 200-triangle mesh (profiles/r2_00_ab.log):
