@@ -287,6 +287,18 @@ typedef struct rt_adaptive_config {
 } rt_adaptive_config;
 RTB_EXPORT int32_t rt_render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac,
                                       double* out_screen, int64_t* out_accum, int32_t* out_samples, rt_stats* stats);
+/* The same adaptive render spread over n_gpus GPUs of this box by ONE host thread of ONE process.  GPU 0 is the device the scene
+ * was committed on, GPUs 1..n-1 are the next visible devices (replicas, as in rt_render_multi).  Every round's paths over the
+ * active list (sample-major, the list's own path space) are cut into n_gpus even ranges, one per GPU, into that GPU's own half
+ * accumulators; at each check point GPU 0 computes the error from the sums of every GPU's A and B, read in place over NVLink
+ * (P2P-mapped pointers; a staged peer copy only where no P2P route exists), compacts the next list and copies it to the others.
+ * Path ids (pixel * max + sample), integer sums and decisions taken from the exact int64 sums make out_accum, out_screen,
+ * out_samples and the path and segment counts bit-identical to rt_render_adaptive for every n_gpus; n_gpus == 1 is
+ * rt_render_adaptive.  Argument rules are rt_render_adaptive's, plus 1 <= n_gpus <= 16 and no more than the
+ * visible devices.  stats: counters summed over the GPUs and the rounds; iterations, ms_device and ms_extend are the slowest
+ * GPU's of each round, summed over the rounds. */
+RTB_EXPORT int32_t rt_render_adaptive_multi(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac, int32_t n_gpus,
+                                            double* out_screen, int64_t* out_accum, int32_t* out_samples, rt_stats* stats);
 #endif
 /* image height the config implies: (image_width as f64 / aspect_ratio) as i32 */
 RTB_EXPORT int32_t RTB_FN(image_height)(const rt_render_config* cfg);

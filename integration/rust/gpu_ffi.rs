@@ -94,6 +94,9 @@ extern "C" {
     /// every pixel until its noise estimate converges, at most cfg.samples_per_pixel; out_samples = W*H per-pixel counts (nullable)
     fn rt_render_adaptive(s: *mut RtScene, cfg: *const RtRenderConfig, ac: *const RtAdaptiveConfig, out_screen: *mut f64, out_accum: *mut i64,
                           out_samples: *mut i32, stats: *mut u8) -> i32;
+    /// rt_render_adaptive with every round's paths spread over n_gpus devices of the box; bit-identical to it for every n_gpus
+    fn rt_render_adaptive_multi(s: *mut RtScene, cfg: *const RtRenderConfig, ac: *const RtAdaptiveConfig, n_gpus: i32, out_screen: *mut f64,
+                                out_accum: *mut i64, out_samples: *mut i32, stats: *mut u8) -> i32;
     fn rt_render_scene_with_time(s: *mut RtScene, t0: f64, t1: f64, path: *const c_char, cfg: *const RtRenderConfig, out_screen: *mut f64, stats: *mut u8) -> i32;
     fn rt_write_ppm(path: *const c_char, screen: *const f64, w: i32, h: i32) -> i32;
 }

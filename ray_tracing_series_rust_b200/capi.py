@@ -139,9 +139,11 @@ DEVICE_SIGNATURES = {
     "peer_timed_out": (C.c_int32, [_P]),
     "peer_destroy": (None, [_P]),
 }
-# rt_render_adaptive, bound on first use (Scene.render_adaptive) like the other product-only controls, so that tools can still load
+# rt_render_adaptive and rt_render_adaptive_multi, bound on first use (Scene.render_adaptive) like the other product-only controls, so that tools can still load
 # builds of the library that predate it side by side (tools/ab_multi.py)
 RENDER_ADAPTIVE_SIGNATURE = (C.c_int32, [_P, C.POINTER(RenderConfig), C.POINTER(AdaptiveConfig), c_d3, C.POINTER(C.c_int64), c_i32p, C.POINTER(Stats)])
+RENDER_ADAPTIVE_MULTI_SIGNATURE = (C.c_int32, [_P, C.POINTER(RenderConfig), C.POINTER(AdaptiveConfig), C.c_int32, c_d3, C.POINTER(C.c_int64), c_i32p,
+                                                C.POINTER(Stats)])
 RT_PEER_HANDLE_BYTES = 64
 RT_SHARD_SAMPLES = 0
 RT_SHARD_TILES = 1
@@ -400,9 +402,10 @@ class Scene:
                                       accum.ctypes.data_as(C.POINTER(C.c_int64)) if want_accum else None, C.byref(st)))
         return screen, accum, st.as_dict()
 
-    def render_adaptive(self, cfg: RenderConfig, threshold: float, min_samples: int = 64, step: int = 16, radius: int = 1):
+    def render_adaptive(self, cfg: RenderConfig, threshold: float, min_samples: int = 64, step: int = 16, radius: int = 1, n_gpus: int = 1):
         """rt_render_adaptive: each pixel rendered until its noise estimate drops below `threshold`, at most cfg.samples_per_pixel
-        samples (include/rtb200.h).  -> (screen[H,W,3] float64, accum[H,W,3] int64, samples[H,W] int32, stats dict)"""
+        samples (include/rtb200.h); n_gpus > 1: rt_render_adaptive_multi, the rounds spread over that many GPUs of this box with the
+        same results.  -> (screen[H,W,3] float64, accum[H,W,3] int64, samples[H,W] int32, stats dict)"""
         H = self.image_height(cfg)
         W = cfg.image_width
         screen = np.zeros((H, W, 3), dtype=np.float64)
@@ -410,10 +413,15 @@ class Scene:
         samples = np.zeros((H, W), dtype=np.int32)
         ac = AdaptiveConfig(int(min_samples), int(step), float(threshold), int(radius))
         st = Stats()
-        fn = self.api.lib.rt_render_adaptive
-        fn.restype, fn.argtypes = RENDER_ADAPTIVE_SIGNATURE
-        self._c(fn(self.h, C.byref(cfg), C.byref(ac), screen.ctypes.data_as(c_d3),
-                                         accum.ctypes.data_as(C.POINTER(C.c_int64)), samples.ctypes.data_as(c_i32p), C.byref(st)))
+        outs = (screen.ctypes.data_as(c_d3), accum.ctypes.data_as(C.POINTER(C.c_int64)), samples.ctypes.data_as(c_i32p), C.byref(st))
+        if n_gpus == 1:
+            fn = self.api.lib.rt_render_adaptive
+            fn.restype, fn.argtypes = RENDER_ADAPTIVE_SIGNATURE
+            self._c(fn(self.h, C.byref(cfg), C.byref(ac), *outs))
+        else:
+            fn = self.api.lib.rt_render_adaptive_multi
+            fn.restype, fn.argtypes = RENDER_ADAPTIVE_MULTI_SIGNATURE
+            self._c(fn(self.h, C.byref(cfg), C.byref(ac), int(n_gpus), *outs))
         return screen, accum, samples, st.as_dict()
 
     def commit_multi(self, n_gpus: int):

@@ -75,14 +75,21 @@ cudaError_t launch_flag_wait(const uint32_t* flag, uint32_t need, uint32_t* time
 cudaError_t launch_reduce_resolve(const AccumShards& shards, int64_t* d_sum_out, uint8_t* d_screen_u8, double* d_screen_f64, int32_t W, int32_t H, int32_t spp,
                                   int32_t rows, cudaStream_t stream);
 
-// ---- adaptive sampling (adaptive.cu, rt_render_adaptive)
+// ---- adaptive sampling (adaptive.cu, rt_render_adaptive / rt_render_adaptive_multi)
+// The half accumulators A and B of every GPU that renders rounds (n = 1: the scene's own GPU); the kernels read them where they lie,
+// like k_reduce_resolve reads AccumShards, and add the int64 components of a pixel before any f64 arithmetic.  Every pointer must be
+// 16-byte aligned: the kernels read pixel pairs and channel pairs with 128-bit loads (A and B of one allocation start at even offsets).
+struct AdaptiveShards {
+    const int64_t* a[RT_MAX_GPUS];
+    const int64_t* b[RT_MAX_GPUS];
+    int32_t n;
+};
 // Check point after n samples (n / 2 in each of the half accumulators A and B) over the active list d_list_in: the half-buffer error of
 // every active pixel into the byte mask d_u (W * rows), its box dilation restricted to the active set into d_keep, the final count n
 // into d_samples for the pixels that leave, and the stable compaction of the pixels that stay into d_list_out; their number is written
 // to *count_out (may be pinned host memory).
 struct AdaptiveCheck {
-    const int64_t* d_a;
-    const int64_t* d_b;
+    AdaptiveShards shards;
     const uint32_t* d_list_in;
     uint32_t n_active;
     uint32_t* d_list_out;
@@ -99,9 +106,9 @@ cudaError_t launch_adaptive_iota(uint32_t* d_list, uint32_t n, cudaStream_t stre
 size_t adaptive_select_temp_bytes(uint32_t max_items);
 cudaError_t launch_adaptive_check(const AdaptiveCheck& c, cudaStream_t stream);
 cudaError_t launch_adaptive_fill(const uint32_t* d_list, uint32_t n_active, int32_t n, int32_t* d_samples, cudaStream_t stream); // samples[list[q]] = n
-// accum_out = A + B, Screen bytes resolved with each pixel's own sample count (0 samples: black)
-cudaError_t launch_resolve_adaptive(const int64_t* d_a, const int64_t* d_b, const int32_t* d_samples, int64_t* d_accum_out, uint8_t* d_screen_u8,
-                                    int32_t W, int32_t H, cudaStream_t stream);
+// accum_out = the sum of every shard's A + B, Screen bytes resolved with each pixel's own sample count (0 samples: black)
+cudaError_t launch_resolve_adaptive(const AdaptiveShards& shards, const int32_t* d_samples, int64_t* d_accum_out, uint8_t* d_screen_u8, int32_t W,
+                                    int32_t H, cudaStream_t stream);
 
 // world.hit for n rays (device pointers)
 cudaError_t launch_trace_batch(const DeviceScene& scene, const rt_ray* d_rays, int64_t n, double t_min, double t_max, int32_t flags, uint64_t seed,

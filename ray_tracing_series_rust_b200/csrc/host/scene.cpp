@@ -9,11 +9,13 @@
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
+#include <condition_variable>
 #include <cstring>
 #include <map>
 #include <memory>
 #include <string>
 #include <mutex>
+#include <system_error>
 #include <thread>
 #include <vector>
 
@@ -153,8 +155,10 @@ struct Replica {
     uint64_t generation = ~0ull;
     DeviceScene scene;
     Workspace* workspace = nullptr;
-    int64_t* d_accum = nullptr;
+    int64_t* d_accum = nullptr; // rt_render_multi's shard; rt_render_adaptive_multi's half accumulators A | B (B at an even offset)
     size_t accum_cap = 0;
+    uint32_t* d_list = nullptr; // rt_render_adaptive_multi: this GPU's copy of the active pixel list
+    size_t list_cap = 0;
     cudaStream_t stream = nullptr;
     bool peer_ok = false; // the gathering GPU can read this arena's accumulator directly
     int64_t* d_stage = nullptr; // on the gathering GPU, only when peer access is unavailable
@@ -165,11 +169,13 @@ struct Replica {
         if (device >= 0) cudaSetDevice(device);
         if (arena) cudaFree(arena);
         if (d_accum) cudaFree(d_accum);
+        if (d_list) cudaFree(d_list);
         if (stream) cudaStreamDestroy(stream);
         free_workspace(workspace);
         cudaSetDevice(cur);
         if (d_stage) cudaFree(d_stage);
-        arena = nullptr; d_accum = nullptr; stream = nullptr; workspace = nullptr; d_stage = nullptr;
+        arena = nullptr; d_accum = nullptr; d_list = nullptr; stream = nullptr; workspace = nullptr; d_stage = nullptr;
+        accum_cap = list_cap = stage_cap = 0;
     }
 };
 
@@ -1499,77 +1505,6 @@ void add_stats(rt_stats& sum, const rt_stats& r, bool concurrent) {
 
 } // namespace
 
-int32_t rt_render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac, double* out_screen, int64_t* out_accum,
-                           int32_t* out_samples, rt_stats* stats) {
-    CHECK_SCENE(s);
-    if (!cfg) return fail(RT_ERR_INVALID, "null config");
-    // argument checks first: they need no committed scene
-    if (!ac) return fail(RT_ERR_INVALID, "null adaptive config");
-    if (ac->step < 1) return fail(RT_ERR_INVALID, "adaptive step < 1");
-    if (!(ac->threshold >= 0.0) || !std::isfinite(ac->threshold)) return fail(RT_ERR_INVALID, "adaptive threshold must be finite and >= 0");
-    if (ac->radius < 0 || ac->radius > 8) return fail(RT_ERR_INVALID, "adaptive radius outside 0..8");
-    if (ac->min_samples < 0 || ac->min_samples > cfg->samples_per_pixel) return fail(RT_ERR_INVALID, "adaptive min_samples outside 0..samples_per_pixel");
-    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
-        return fail(RT_ERR_INVALID, "rt_render_adaptive takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
-    if (cfg->sample_begin != 0 || (cfg->sample_end != 0 && cfg->sample_end != cfg->samples_per_pixel))
-        return fail(RT_ERR_INVALID, "rt_render_adaptive renders every sample range itself: sample_begin / sample_end must cover [0, samples_per_pixel)");
-    RenderJob job;
-    int32_t rc = make_job(s, cfg, job);
-    if (rc != RT_OK) return rc;
-    const auto t0 = std::chrono::steady_clock::now();
-    DeviceGuard guard(s->dev.device);
-    const size_t npix = (size_t)job.width * job.height, n = npix * 3;
-    if ((rc = ensure_out_buffers(s, n)) != RT_OK) return rc;
-    if ((rc = ensure_adaptive_buffers(s, npix)) != RT_OK) return rc;
-    RenderBuffers& o = s->out;
-    AdaptiveBuffers& b = s->adaptive;
-    const RenderTuning tune = tuning_for(s, cfg);
-    const int32_t max = job.spp_total, step = ac->step;
-    const uint32_t rendered = (uint32_t)job.width * (uint32_t)job.rows;
-    cudaError_t e;
-    if ((e = cudaMemsetAsync(b.d_a, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess || (e = cudaMemsetAsync(b.d_b, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess ||
-        (e = cudaMemsetAsync(b.d_samples, 0, npix * sizeof(int32_t), o.stream)) != cudaSuccess || (e = launch_adaptive_iota(b.d_list[0], rendered, o.stream)) != cudaSuccess)
-        return fail_cuda(e, "adaptive set-up");
-    rt_stats sum;
-    std::memset(&sum, 0, sizeof sum);
-    uint32_t n_active = rendered;
-    int cur = 0;
-    for (int64_t k = 0; n_active > 0 && k * step < max; ++k) {
-        const int32_t s0 = (int32_t)(k * step), s1 = (int32_t)std::min<int64_t>((k + 1) * step, max);
-        RenderJob rj = job;
-        rj.sample_begin = s0; rj.sample_end = s1;
-        rj.d_pixels = b.d_list[cur]; rj.n_pixels = n_active;
-        rt_stats rs;
-        std::memset(&rs, 0, sizeof rs);
-        if ((e = launch_render(s->dev.scene, rj, tune, (k & 1) ? b.d_b : b.d_a, o.stream, &rs, &s->workspace)) != cudaSuccess) return fail_cuda(e, "adaptive render round");
-        add_stats(sum, rs, false);
-        if (!(k & 1) || s1 < ac->min_samples || s1 >= max) continue;
-        AdaptiveCheck c;
-        c.d_a = b.d_a; c.d_b = b.d_b;
-        c.d_list_in = b.d_list[cur]; c.n_active = n_active; c.d_list_out = b.d_list[cur ^ 1]; c.count_out = b.h_count;
-        c.d_u = b.d_u; c.d_keep = b.d_keep; c.d_samples = b.d_samples;
-        c.d_temp = b.d_temp; c.temp_bytes = b.temp_bytes;
-        c.W = job.width; c.rows = job.rows; c.n = s1; c.radius = ac->radius; c.threshold = ac->threshold;
-        if ((e = launch_adaptive_check(c, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive check");
-        if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive check sync");
-        n_active = *b.h_count;
-        cur ^= 1;
-    }
-    if ((e = launch_adaptive_fill(b.d_list[cur], n_active, max, b.d_samples, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive counts");
-    if ((e = launch_resolve_adaptive(b.d_a, b.d_b, b.d_samples, o.d_accum, o.d_u8, job.width, job.height, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive resolve");
-    if (out_screen && (e = cudaMemcpyAsync(o.h_u8, o.d_u8, n, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "screen copy");
-    if (out_accum && (e = cudaMemcpyAsync(out_accum, o.d_accum, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "accum copy");
-    if (out_samples && (e = cudaMemcpyAsync(out_samples, b.d_samples, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
-        return fail_cuda(e, "samples copy");
-    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive sync");
-    if (out_screen) widen_screen(o.h_u8, out_screen, n);
-    if (stats) {
-        *stats = sum;
-        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    }
-    return RT_OK;
-}
-
 // ---- multi-GPU inside the library (SURVEY.md 8(b) n_gpus / shard_mode, 8(e)): one process, N devices
 namespace {
 
@@ -1731,6 +1666,239 @@ int32_t rt_render_multi(rt_scene* s, const rt_render_config* cfg, int32_t n_gpus
         stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     }
     return RT_OK;
+}
+
+// ---- adaptive sampling on one GPU or several (rt_render_adaptive, rt_render_adaptive_multi)
+namespace {
+
+// Where the render threads of rt_render_adaptive_multi meet once per check point.  The workers (GPUs 1..n-1) arrive when their rounds
+// up to the check point have drained and wait until the calling thread (GPU 0) has run the check and handed out the next list.
+// fail() lets every thread go for good: the first error anywhere ends the call without leaving a thread waiting.
+class RoundBarrier {
+  public:
+    explicit RoundBarrier(int workers) : workers_(workers) {}
+    bool arrive_and_wait() { // worker; false: stop
+        std::unique_lock<std::mutex> lk(m_);
+        if (failed_) return false;
+        const uint64_t gen = gen_;
+        ++arrived_;
+        cv_.notify_all();
+        cv_.wait(lk, [&] { return gen_ != gen || failed_; });
+        return !failed_;
+    }
+    bool gather() { // GPU 0; false: a worker failed
+        std::unique_lock<std::mutex> lk(m_);
+        cv_.wait(lk, [&] { return arrived_ == workers_ || failed_; });
+        return !failed_;
+    }
+    void release() {
+        std::lock_guard<std::mutex> lk(m_);
+        arrived_ = 0;
+        ++gen_;
+        cv_.notify_all();
+    }
+    void fail() {
+        std::lock_guard<std::mutex> lk(m_);
+        failed_ = true;
+        cv_.notify_all();
+    }
+    bool failed() {
+        std::lock_guard<std::mutex> lk(m_);
+        return failed_;
+    }
+
+  private:
+    std::mutex m_;
+    std::condition_variable cv_;
+    int workers_, arrived_ = 0;
+    uint64_t gen_ = 0;
+    bool failed_ = false;
+};
+
+// The rounds of rt_render_adaptive spread over n_gpus GPUs (n_gpus = 1: the scene's own GPU only, with the launches of a plain
+// single-GPU render).  GPU g renders the g-th of n_gpus even ranges of each round's paths (sample-major over the active list) into its
+// own A or B, on its own host thread; GPU 0 runs the check points and the resolve over every GPU's A and B.
+int32_t render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac, int32_t n_gpus, double* out_screen,
+                        int64_t* out_accum, int32_t* out_samples, rt_stats* stats) {
+    CHECK_SCENE(s);
+    if (!cfg) return fail(RT_ERR_INVALID, "null config");
+    // argument checks first: they need no committed scene
+    if (!ac) return fail(RT_ERR_INVALID, "null adaptive config");
+    if (ac->step < 1) return fail(RT_ERR_INVALID, "adaptive step < 1");
+    if (!(ac->threshold >= 0.0) || !std::isfinite(ac->threshold)) return fail(RT_ERR_INVALID, "adaptive threshold must be finite and >= 0");
+    if (ac->radius < 0 || ac->radius > 8) return fail(RT_ERR_INVALID, "adaptive radius outside 0..8");
+    if (ac->min_samples < 0 || ac->min_samples > cfg->samples_per_pixel) return fail(RT_ERR_INVALID, "adaptive min_samples outside 0..samples_per_pixel");
+    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
+        return fail(RT_ERR_INVALID, "rt_render_adaptive takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
+    if (cfg->sample_begin != 0 || (cfg->sample_end != 0 && cfg->sample_end != cfg->samples_per_pixel))
+        return fail(RT_ERR_INVALID, "rt_render_adaptive renders every sample range itself: sample_begin / sample_end must cover [0, samples_per_pixel)");
+    if (n_gpus < 1 || n_gpus > RT_MAX_GPUS) return fail(RT_ERR_INVALID, "n_gpus outside 1..16");
+    RenderJob job;
+    int32_t rc = make_job(s, cfg, job);
+    if (rc != RT_OK) return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    DeviceGuard guard(s->dev.device);
+    const size_t npix = (size_t)job.width * job.height, n = npix * 3;
+    // A replica's B starts nb elements after its A: an even offset keeps B 16-byte aligned for the kernels' 128-bit loads when n is odd
+    const size_t nb = (n + 1) & ~(size_t)1;
+    if ((rc = ensure_out_buffers(s, n)) != RT_OK) return rc;
+    if ((rc = ensure_adaptive_buffers(s, npix)) != RT_OK) return rc;
+    if (n_gpus > 1) {
+        if ((rc = ensure_replicas(s, n_gpus, 2 * nb)) != RT_OK) return rc; // d_accum = A | B, d_stage (no P2P route) as large
+        for (int g = 1; g < n_gpus; ++g) {
+            Replica& r = s->replicas[(size_t)g - 1];
+            if (npix <= r.list_cap) continue;
+            cudaError_t e;
+            if ((e = cudaSetDevice(r.device)) == cudaSuccess) {
+                if (r.d_list) cudaFree(r.d_list);
+                r.d_list = nullptr; r.list_cap = 0;
+                e = cudaMalloc(&r.d_list, npix * sizeof(uint32_t));
+            }
+            cudaSetDevice(s->dev.device);
+            if (e != cudaSuccess) return fail_cuda(e, "replica pixel list");
+            r.list_cap = npix;
+        }
+    }
+    RenderBuffers& o = s->out;
+    AdaptiveBuffers& b = s->adaptive;
+    const RenderTuning tune = tuning_for(s, cfg);
+    const int32_t max = job.spp_total, step = ac->step;
+    const uint32_t rendered = (uint32_t)job.width * (uint32_t)job.rows;
+    cudaError_t e;
+    if ((e = cudaMemsetAsync(b.d_a, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess || (e = cudaMemsetAsync(b.d_b, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess ||
+        (e = cudaMemsetAsync(b.d_samples, 0, npix * sizeof(int32_t), o.stream)) != cudaSuccess || (e = launch_adaptive_iota(b.d_list[0], rendered, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "adaptive set-up");
+
+    // every GPU's A and B as GPU 0 reads them: in place (its own, P2P-mapped peers, alias mode) or copied into staging next to it
+    auto shards = [&](AdaptiveShards& sh) -> cudaError_t {
+        std::memset(&sh, 0, sizeof sh);
+        sh.n = n_gpus;
+        sh.a[0] = b.d_a; sh.b[0] = b.d_b;
+        for (int g = 1; g < n_gpus; ++g) {
+            Replica& r = s->replicas[(size_t)g - 1];
+            const int64_t* ab = r.d_accum;
+            if (!r.peer_ok) {
+                const cudaError_t ce = cudaMemcpyPeerAsync(r.d_stage, s->dev.device, r.d_accum, r.device, 2 * nb * sizeof(int64_t), o.stream);
+                if (ce != cudaSuccess) return ce;
+                ab = r.d_stage;
+            }
+            sh.a[g] = ab; sh.b[g] = ab + nb;
+        }
+        return cudaSuccess;
+    };
+
+    std::vector<std::vector<rt_stats>> st((size_t)n_gpus); // [GPU][round]
+    std::vector<cudaError_t> errs((size_t)n_gpus, cudaSuccess);
+    std::vector<const char*> what((size_t)n_gpus, "");
+    RoundBarrier bar(n_gpus - 1);
+    uint32_t n_active = rendered; // written by GPU 0 at a check point, read by the workers once the barrier lets them go
+    int cur = 0;                  // GPU 0's current list (b.d_list[cur]); the workers' is r.d_list
+    auto run = [&](int g) {
+        Replica* r = g ? &s->replicas[(size_t)g - 1] : nullptr;
+        cudaStream_t stream = r ? r->stream : o.stream;
+        int64_t* A = r ? r->d_accum : b.d_a;
+        int64_t* B = r ? r->d_accum + nb : b.d_b;
+        cudaError_t& err = errs[(size_t)g];
+        auto stop = [&](cudaError_t ce, const char* w) { err = ce; what[(size_t)g] = w; bar.fail(); };
+        if (r && ((err = cudaSetDevice(r->device)) != cudaSuccess || (err = cudaMemsetAsync(r->d_accum, 0, 2 * nb * sizeof(int64_t), stream)) != cudaSuccess ||
+                  (err = launch_adaptive_iota(r->d_list, rendered, stream)) != cudaSuccess))
+            return stop(err, "adaptive set-up");
+        uint32_t na = rendered;
+        for (int64_t k = 0; na > 0 && k * step < max; ++k) {
+            if (n_gpus > 1 && bar.failed()) return;
+            const int32_t s0 = (int32_t)(k * step), s1 = (int32_t)std::min<int64_t>((k + 1) * step, max);
+            RenderJob rj = job;
+            rj.sample_begin = s0; rj.sample_end = s1;
+            rj.d_pixels = r ? r->d_list : b.d_list[cur]; rj.n_pixels = na;
+            // an even share of the round's paths: balanced in every round, consecutive paths on neighbouring pixels
+            const uint64_t T = (uint64_t)na * (uint64_t)(s1 - s0);
+            rj.path_begin = T * (uint64_t)g / (uint64_t)n_gpus;
+            rj.path_end = T * (uint64_t)(g + 1) / (uint64_t)n_gpus;
+            rt_stats rs;
+            std::memset(&rs, 0, sizeof rs);
+            if (rj.path_end > rj.path_begin) { // an empty range renders nothing (more GPUs than paths)
+                const DeviceScene& scene = r ? r->scene : s->dev.scene;
+                if ((err = launch_render(scene, rj, tune, (k & 1) ? B : A, stream, &rs, r ? &r->workspace : &s->workspace)) != cudaSuccess)
+                    return stop(err, "adaptive render round");
+            }
+            st[(size_t)g].push_back(rs);
+            if (!(k & 1) || s1 < ac->min_samples || s1 >= max) continue;
+            if (r) { // launch_render has drained the stream, except where the range was empty: the set-up may still be in flight
+                if ((err = cudaStreamSynchronize(stream)) != cudaSuccess) return stop(err, "adaptive round sync");
+                if (!bar.arrive_and_wait()) return;
+                na = n_active;
+                continue;
+            }
+            if (!bar.gather()) return;
+            AdaptiveCheck c;
+            if ((err = shards(c.shards)) != cudaSuccess) return stop(err, "peer copy");
+            c.d_list_in = b.d_list[cur]; c.n_active = na; c.d_list_out = b.d_list[cur ^ 1]; c.count_out = b.h_count;
+            c.d_u = b.d_u; c.d_keep = b.d_keep; c.d_samples = b.d_samples;
+            c.d_temp = b.d_temp; c.temp_bytes = b.temp_bytes;
+            c.W = job.width; c.rows = job.rows; c.n = s1; c.radius = ac->radius; c.threshold = ac->threshold;
+            if ((err = launch_adaptive_check(c, o.stream)) != cudaSuccess) return stop(err, "adaptive check");
+            if ((err = cudaStreamSynchronize(o.stream)) != cudaSuccess) return stop(err, "adaptive check sync");
+            na = n_active = *b.h_count;
+            cur ^= 1;
+            if (n_gpus > 1) {
+                for (int h = 1; h < n_gpus && na > 0; ++h) {
+                    Replica& rh = s->replicas[(size_t)h - 1];
+                    if ((err = cudaMemcpyPeerAsync(rh.d_list, rh.device, b.d_list[cur], s->dev.device, na * sizeof(uint32_t), o.stream)) != cudaSuccess)
+                        return stop(err, "pixel list copy");
+                }
+                if ((err = cudaStreamSynchronize(o.stream)) != cudaSuccess) return stop(err, "pixel list copy sync");
+                bar.release();
+            }
+        }
+        if (r && (err = cudaStreamSynchronize(stream)) != cudaSuccess) return stop(err, "adaptive round sync");
+    };
+    {
+        std::vector<std::thread> pool;
+        bool started = true;
+        try {
+            for (int g = 1; g < n_gpus; ++g) pool.emplace_back(run, g);
+        } catch (const std::system_error&) {
+            started = false;
+            bar.fail();
+        }
+        if (started) run(0); // the calling thread is GPU 0
+        for (std::thread& th : pool) th.join();
+        if (!started) return fail(RT_ERR_CUDA, "could not start the render threads");
+    }
+    for (int g = 0; g < n_gpus; ++g)
+        if (errs[(size_t)g] != cudaSuccess) return fail_cuda(errs[(size_t)g], what[(size_t)g]);
+    AdaptiveShards sh;
+    if ((e = launch_adaptive_fill(b.d_list[cur], n_active, max, b.d_samples, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive counts");
+    if ((e = shards(sh)) != cudaSuccess) return fail_cuda(e, "peer copy");
+    if ((e = launch_resolve_adaptive(sh, b.d_samples, o.d_accum, o.d_u8, job.width, job.height, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive resolve");
+    if (out_screen && (e = cudaMemcpyAsync(o.h_u8, o.d_u8, n, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "screen copy");
+    if (out_accum && (e = cudaMemcpyAsync(out_accum, o.d_accum, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "accum copy");
+    if (out_samples && (e = cudaMemcpyAsync(out_samples, b.d_samples, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "samples copy");
+    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive sync");
+    if (out_screen) widen_screen(o.h_u8, out_screen, n);
+    if (stats) { // the GPUs of a round run at the same time, the rounds one after the other
+        std::memset(stats, 0, sizeof *stats);
+        for (size_t k = 0; k < st[0].size(); ++k) {
+            rt_stats round = st[0][k];
+            for (int g = 1; g < n_gpus; ++g) add_stats(round, st[(size_t)g][k], true);
+            add_stats(*stats, round, false);
+        }
+        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    return RT_OK;
+}
+
+} // namespace
+
+int32_t rt_render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac, double* out_screen, int64_t* out_accum,
+                           int32_t* out_samples, rt_stats* stats) {
+    return render_adaptive(s, cfg, ac, 1, out_screen, out_accum, out_samples, stats);
+}
+
+int32_t rt_render_adaptive_multi(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac, int32_t n_gpus, double* out_screen,
+                                 int64_t* out_accum, int32_t* out_samples, rt_stats* stats) {
+    return render_adaptive(s, cfg, ac, n_gpus, out_screen, out_accum, out_samples, stats);
 }
 
 // ---- peer group: the exchange of the one-process-per-GPU layout without a collective library on the data path
