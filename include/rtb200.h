@@ -300,6 +300,45 @@ RTB_EXPORT int32_t rt_render_adaptive(rt_scene* s, const rt_render_config* cfg, 
 RTB_EXPORT int32_t rt_render_adaptive_multi(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac, int32_t n_gpus,
                                             double* out_screen, int64_t* out_accum, int32_t* out_samples, rt_stats* stats);
 #endif
+
+/* First-hit feature buffers of the render's own paths.  For every pixel of a rendered row and every sample s of cfg's range
+ * [sample_begin, sample_end): the path's camera ray (pixel jitter, lens, shutter: exactly rt_render's path id pixel*spp + s),
+ * ONE world.hit(ray, 0.001, inf) with media sampled from the path's keyed stream at segment 0 (= the render's first hit), then
+ *   Lambertian / Isotropic : albedo = Texture::value(u, v, p)         normal = rec.normal (Isotropic: 0)
+ *   Metal                  : albedo = Metal.albedo                    normal = rec.normal
+ *   Dielectric             : albedo = (1, 1, 1)                       normal = rec.normal
+ *   DiffuseLight           : albedo = clamp(emitted(u, v, p), 0, 1)   normal = rec.normal
+ *   miss                   : albedo = clamp(background or sky, 0, 1)  normal = 0
+ * out_albedo / out_normal (W*H*3 int64, nullable): per-pixel sums of round-to-nearest-even(x * 2^32); rows >= the rendered rows
+ * stay 0.  Mode flags are ignored (one kernel); a tile shard (count > 1) and RT_RENDER_NO_WAIT are RT_ERR_INVALID.
+ * stats: paths = segments = rays traced.  The oracle's side is built by the tests (tests/oracle_aov). */
+RTB_EXPORT int32_t RTB_FN(render_aov)(rt_scene* s, const rt_render_config* cfg, int64_t* out_albedo, int64_t* out_normal, rt_stats* stats);
+
+#ifndef RTB_PREFIX_ORC
+/* A denoised render (DESIGN.md section 11; the numpy reference is ray_tracing_series_rust_b200/denoise.py).  With n = samples_per_pixel
+ * and hA = n / 2: samples [0, hA) are rendered into a half accumulator A and [hA, n) into B (out_accum = A + B = rt_render's
+ * out_accum bit for bit), the feature sums of samples [0, aov_samples) as rt_render_aov, then `iterations` passes of a feature-guided
+ * a-trous filter (steps 1, 2, 4, ...) in f64 over the rendered rows, starting from c = mean, v = (lum(A mean) - lum(B mean))^2 hA hB / n^2:
+ *   vbar = 3x3 blur of v (1/4, 1/2, 1/4 per axis, valid taps renormalised)
+ *   w(q) = h(dx) h(dy) exp(-(|lum(c_p) - lum(c_q)| / (sigma_color sqrt(vbar_p) + 1e-10) + |a_p - a_q|^2 / sigma_albedo^2 + |n_p - n_q|^2 / sigma_normal^2))
+ *   over the 25 taps q = p + step (dx, dy), dx, dy in -2..2, h = (1/16, 1/4, 3/8, 1/4, 1/16);  c' = sum w c_q / sum w,  v' = sum w^2 v_q / (sum w)^2
+ * lum(x) = (0.2126 r + 0.7152 g) + 0.0722 b; a, n = the feature means (the mean normal is not renormalised).  out_linear (W*H*3
+ * doubles, Screen layout) = the filtered mean, out_screen = its Screen values (rt_render's quantisation); rows >= the rendered rows
+ * stay 0.  Integer sums and a gather without atomics make every output identical in every render mode and on every run.
+ * cfg must render the whole [0, samples_per_pixel) with samples_per_pixel >= 2, without a tile shard (count > 1) and without
+ * RT_RENDER_NO_WAIT; the mode flags apply to both half renders.  stats: the half renders' counters summed; kernel_launches also
+ * counts the feature pass and the filter kernels. */
+typedef struct rt_denoise_config {
+    int32_t aov_samples;  /* 1 .. samples_per_pixel: features from the render's samples [0, aov_samples) */
+    int32_t iterations;   /* 1 .. 8: a-trous passes, steps 1, 2, 4, ... */
+    double sigma_color;   /* > 0, finite: luminance edge stop, in units of the pixel's noise standard deviation */
+    double sigma_albedo;  /* > 0, finite */
+    double sigma_normal;  /* > 0, finite */
+} rt_denoise_config;
+RTB_EXPORT int32_t rt_render_denoised(rt_scene* s, const rt_render_config* cfg, const rt_denoise_config* dc,
+                                      double* out_screen /* denoised Screen, nullable */, double* out_linear /* nullable */,
+                                      int64_t* out_accum /* nullable: == rt_render's out_accum */, rt_stats* stats);
+#endif
 /* image height the config implies: (image_width as f64 / aspect_ratio) as i32 */
 RTB_EXPORT int32_t RTB_FN(image_height)(const rt_render_config* cfg);
 

@@ -54,6 +54,16 @@ pub struct RtAdaptiveConfig {
     pub radius: i32,      // 0..=8: a pixel stays active while an unconverged pixel is this close
 }
 
+/// rt_denoise_config (include/rtb200.h): the filter of rt_render_denoised
+#[repr(C)]
+pub struct RtDenoiseConfig {
+    pub aov_samples: i32,  // 1 ..= samples_per_pixel: features from the render's samples [0, aov_samples)
+    pub iterations: i32,   // 1 ..= 8: a-trous passes, steps 1, 2, 4, ...
+    pub sigma_color: f64,  // > 0, finite: luminance edge stop, in units of the pixel's noise standard deviation
+    pub sigma_albedo: f64, // > 0, finite
+    pub sigma_normal: f64, // > 0, finite
+}
+
 #[link(name = "rtb200")]
 extern "C" {
     fn rt_scene_create() -> *mut RtScene;
@@ -97,6 +107,11 @@ extern "C" {
     /// rt_render_adaptive with every round's paths spread over n_gpus devices of the box; bit-identical to it for every n_gpus
     fn rt_render_adaptive_multi(s: *mut RtScene, cfg: *const RtRenderConfig, ac: *const RtAdaptiveConfig, n_gpus: i32, out_screen: *mut f64,
                                 out_accum: *mut i64, out_samples: *mut i32, stats: *mut u8) -> i32;
+    /// first-hit albedo / normal sums (round(x * 2^32)) of the render's paths over cfg's sample range; W*H*3 each, nullable
+    fn rt_render_aov(s: *mut RtScene, cfg: *const RtRenderConfig, out_albedo: *mut i64, out_normal: *mut i64, stats: *mut u8) -> i32;
+    /// two half renders + features + a-trous filter: out_screen = denoised Screen, out_linear = filtered mean, out_accum = rt_render's
+    fn rt_render_denoised(s: *mut RtScene, cfg: *const RtRenderConfig, dc: *const RtDenoiseConfig, out_screen: *mut f64, out_linear: *mut f64,
+                          out_accum: *mut i64, stats: *mut u8) -> i32;
     fn rt_render_scene_with_time(s: *mut RtScene, t0: f64, t1: f64, path: *const c_char, cfg: *const RtRenderConfig, out_screen: *mut f64, stats: *mut u8) -> i32;
     fn rt_write_ppm(path: *const c_char, screen: *const f64, w: i32, h: i32) -> i32;
 }

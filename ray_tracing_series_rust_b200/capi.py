@@ -65,6 +65,17 @@ class AdaptiveConfig(C.Structure):
     ]
 
 
+class DenoiseConfig(C.Structure):
+    """rt_denoise_config (rt_render_denoised)"""
+    _fields_ = [
+        ("aov_samples", C.c_int32),
+        ("iterations", C.c_int32),
+        ("sigma_color", C.c_double),
+        ("sigma_albedo", C.c_double),
+        ("sigma_normal", C.c_double),
+    ]
+
+
 RAY_DTYPE = np.dtype([("o", "<f8", 3), ("d", "<f8", 3), ("time", "<f8")], align=True)
 HIT_DTYPE = np.dtype(
     [("prim_id", "<i4"), ("mat_id", "<i4"), ("t", "<f8"), ("p", "<f8", 3), ("normal", "<f8", 3),
@@ -144,6 +155,9 @@ DEVICE_SIGNATURES = {
 RENDER_ADAPTIVE_SIGNATURE = (C.c_int32, [_P, C.POINTER(RenderConfig), C.POINTER(AdaptiveConfig), c_d3, C.POINTER(C.c_int64), c_i32p, C.POINTER(Stats)])
 RENDER_ADAPTIVE_MULTI_SIGNATURE = (C.c_int32, [_P, C.POINTER(RenderConfig), C.POINTER(AdaptiveConfig), C.c_int32, c_d3, C.POINTER(C.c_int64), c_i32p,
                                                 C.POINTER(Stats)])
+# rt_render_aov (both libraries) and rt_render_denoised, bound on first use like rt_render_adaptive
+RENDER_AOV_SIGNATURE = (C.c_int32, [_P, C.POINTER(RenderConfig), C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(Stats)])
+RENDER_DENOISED_SIGNATURE = (C.c_int32, [_P, C.POINTER(RenderConfig), C.POINTER(DenoiseConfig), c_d3, c_d3, C.POINTER(C.c_int64), C.POINTER(Stats)])
 RT_PEER_HANDLE_BYTES = 64
 RT_SHARD_SAMPLES = 0
 RT_SHARD_TILES = 1
@@ -423,6 +437,43 @@ class Scene:
             fn.restype, fn.argtypes = RENDER_ADAPTIVE_MULTI_SIGNATURE
             self._c(fn(self.h, C.byref(cfg), C.byref(ac), int(n_gpus), *outs))
         return screen, accum, samples, st.as_dict()
+
+    def render_aov(self, cfg: RenderConfig, raw: bool = False):
+        """rt_render_aov: first-hit albedo and normal of the render's paths over cfg's sample range [sample_begin, sample_end)
+        (include/rtb200.h).  -> (albedo[H,W,3], normal[H,W,3], stats dict): the means as float64, or with raw=True the int64 sums
+        of round(x * 2^32)."""
+        H = self.image_height(cfg)
+        W = cfg.image_width
+        albedo = np.zeros((H, W, 3), dtype=np.int64)
+        normal = np.zeros((H, W, 3), dtype=np.int64)
+        st = Stats()
+        fn = getattr(self.api.lib, self.api.prefix + "render_aov")
+        fn.restype, fn.argtypes = RENDER_AOV_SIGNATURE
+        self._c(fn(self.h, C.byref(cfg), albedo.ctypes.data_as(C.POINTER(C.c_int64)), normal.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(st)))
+        if raw:
+            return albedo, normal, st.as_dict()
+        m = (cfg.sample_end or cfg.samples_per_pixel) - cfg.sample_begin
+        return albedo / ACCUM_SCALE / m, normal / ACCUM_SCALE / m, st.as_dict()
+
+    def render_denoised(self, cfg: RenderConfig, aov_samples: int | None = None, iterations: int = 5, sigma_color: float = 4.0,
+                        sigma_albedo: float = 0.1, sigma_normal: float = 0.125):
+        """rt_render_denoised: two half renders, the feature pass over samples [0, aov_samples) (default min(8, spp)) and the
+        feature-guided a-trous filter (include/rtb200.h, DESIGN.md section 11).
+        -> (screen[H,W,3] float64 denoised Screen, linear[H,W,3] float64 filtered mean, accum[H,W,3] int64 = rt_render's, stats dict)"""
+        H = self.image_height(cfg)
+        W = cfg.image_width
+        if aov_samples is None:
+            aov_samples = min(8, cfg.samples_per_pixel)
+        screen = np.zeros((H, W, 3), dtype=np.float64)
+        linear = np.zeros((H, W, 3), dtype=np.float64)
+        accum = np.zeros((H, W, 3), dtype=np.int64)
+        dc = DenoiseConfig(int(aov_samples), int(iterations), float(sigma_color), float(sigma_albedo), float(sigma_normal))
+        st = Stats()
+        fn = self.api.lib.rt_render_denoised
+        fn.restype, fn.argtypes = RENDER_DENOISED_SIGNATURE
+        self._c(fn(self.h, C.byref(cfg), C.byref(dc), screen.ctypes.data_as(c_d3), linear.ctypes.data_as(c_d3),
+                   accum.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(st)))
+        return screen, linear, accum, st.as_dict()
 
     def commit_multi(self, n_gpus: int):
         return self._c(self.api.scene_commit_multi(self.h, int(n_gpus)))

@@ -10,6 +10,7 @@
 #include <cstdint>
 
 #include "kernels.h"
+#include "rt_device.cuh"
 
 namespace rtb {
 
@@ -100,10 +101,7 @@ __global__ void __launch_bounds__(256) k_resolve_adaptive(const AdaptiveShards H
             double out = 0.0;
             if (np > 0) {
                 const double sum = (double)s[k] * (1.0 / 4294967296.0);
-                double c = sqrt(sum * (1.0 / (double)np));
-                c = c < 0.0 ? 0.0 : (c > 1.0 ? 1.0 : c);     // mutil.rs:1-9 (NaN passes through)
-                const double q = 255.9 * c;
-                out = (q != q) ? 0.0 : (double)(int32_t)q;    // `as i32`: truncation, NaN -> 0
+                out = screen_value(sum * (1.0 / (double)np));
             }
             accum_out[e] = s[k];
             screen_u8[e] = (uint8_t)out;

@@ -1138,10 +1138,7 @@ __global__ void k_resolve(const int64_t* __restrict__ accum, double* __restrict_
         if (j < rows) {
             const double sum = (double)accum[i] * (1.0 / 4294967296.0);
             const double scale = 1.0 / (double)spp;
-            double c = sqrt(sum * scale);
-            c = c < 0.0 ? 0.0 : (c > 1.0 ? 1.0 : c);     // mutil.rs:1-9 (NaN passes through)
-            const double q = 255.9 * c;
-            out = (q != q) ? 0.0 : (double)(int32_t)q;    // `as i32`: truncation, NaN -> 0
+            out = screen_value(sum * scale);
         }
         screen[i] = out;
     }
@@ -1201,10 +1198,7 @@ __global__ void __launch_bounds__(256) k_reduce_resolve(const AccumShards A, int
             double out = 0.0;
             if (e < rendered) { // rows >= `rows` stay (0,0,0): world.rs:1198-1202
                 const double sum = (double)(k ? s1 : s0) * (1.0 / 4294967296.0);
-                double c = sqrt(sum * scale);
-                c = c < 0.0 ? 0.0 : (c > 1.0 ? 1.0 : c);     // mutil.rs:1-9 (NaN passes through)
-                const double q = 255.9 * c;
-                out = (q != q) ? 0.0 : (double)(int32_t)q;    // `as i32`: truncation, NaN -> 0
+                out = screen_value(sum * scale);
             }
             if (screen_u8) screen_u8[e] = (uint8_t)out;
             if (screen_f64) screen_f64[e] = out;

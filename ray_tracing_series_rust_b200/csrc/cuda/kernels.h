@@ -110,6 +110,31 @@ cudaError_t launch_adaptive_fill(const uint32_t* d_list, uint32_t n_active, int3
 cudaError_t launch_resolve_adaptive(const AdaptiveShards& shards, const int32_t* d_samples, int64_t* d_accum_out, uint8_t* d_screen_u8, int32_t W,
                                     int32_t H, cudaStream_t stream);
 
+// ---- denoised renders (denoise.cu, rt_render_aov / rt_render_denoised)
+// First-hit feature sums of the job's paths (its rows, its samples [sample_begin, sample_end), path id pixel * spp_total + sample):
+// round-to-nearest-even(x * 2^32) added into d_albedo / d_normal (W*H*3 int64 each, nullable, zeroed by the caller).  Walks the 4-wide
+// tree where the scene carries one.
+cudaError_t launch_aov(const DeviceScene& scene, const RenderJob& job, int64_t* d_albedo, int64_t* d_normal, cudaStream_t stream);
+// The feature-guided a-trous filter of rt_render_denoised over the half accumulators A (hA samples) and B (hB) and the feature sums
+// of m samples.  Device buffers: c[2] (W*H*3 f64), v[2] and vbar (W*H f64), feat (W*H*6 f64) are scratch; accum_out (nullable) = A + B,
+// linear_out (nullable, W*H*3 f64) = the filtered mean, screen_u8 (nullable) = its Screen bytes.  Rows >= rows are 0 in every output.
+struct DenoiseJob {
+    const int64_t* a;
+    const int64_t* b;
+    const int64_t* albedo;
+    const int64_t* normal;
+    int32_t W, H, rows, hA, hB, m, iterations;
+    double sigma_color, sigma_albedo, sigma_normal;
+    double* c[2];
+    double* v[2];
+    double* vbar;
+    double* feat;
+    int64_t* accum_out;
+    double* linear_out;
+    uint8_t* screen_u8;
+};
+cudaError_t launch_denoise(const DenoiseJob& j, cudaStream_t stream);
+
 // world.hit for n rays (device pointers)
 cudaError_t launch_trace_batch(const DeviceScene& scene, const rt_ray* d_rays, int64_t n, double t_min, double t_max, int32_t flags, uint64_t seed,
                                rt_hit* d_out, cudaStream_t stream);

@@ -1232,4 +1232,43 @@ template <class G> RT_DEV Ray camera_first_ray(const DCamera& c, int32_t ii, int
     return r;
 }
 
+// ------------------------------------------------------------------ Screen value of one channel (vec3.rs:89-107)
+// mean = sum / samples; the reference's gamma 2 (sqrt), clamp to [0, 1] (mutil.rs:1-9, NaN passes through), `(255.9 * c) as i32`
+// (truncation, NaN -> 0).  Every resolve kernel quantises through this one function.
+RT_DEV double screen_value(double mean) {
+    double c = sqrt(mean);
+    c = c < 0.0 ? 0.0 : (c > 1.0 ? 1.0 : c);
+    const double q = 255.9 * c;
+    return (q != q) ? 0.0 : (double)(int32_t)q;
+}
+
+// ------------------------------------------------------------------ first-hit feature buffers (rt_render_aov, denoise.cu k_aov)
+// Path path_id of pixel (ii, j): its camera ray, then ONE world.hit(ray, 0.001, inf) with media sampled from the path's keyed stream
+// at segment 0 - the render's own first hit.  albedo: Lambertian / Isotropic Texture::value, Metal albedo, Dielectric 1, DiffuseLight
+// emitted clamped to [0, 1]; a miss: the background (or sky) clamped to [0, 1].  normal: HitRecord.normal, 0 for media and misses.
+RT_DEV double clamp01(double x) { return x < 0.0 ? 0.0 : (x > 1.0 ? 1.0 : x); }
+template <bool WIDE>
+RT_DEV void aov_path(const DeviceScene& S, int32_t ii, int32_t j, int32_t W, int32_t H, uint64_t seed, uint64_t path_id, D3& albedo, D3& normal) {
+    uint32_t draw = 0;
+    const Ray r = camera_first_ray<PathRng>(S.cam, ii, j, W, H, seed, path_id, draw);
+    HitRec h;
+    if (!world_hit<false, 1, true, true, RT_PM_ALL, true, WIDE>(S, r, 0.001, RT_INF, true, seed, path_id, 0u, h, nullptr)) {
+        const F3 bg = miss_color(S, r.d);
+        albedo = mk3(clamp01(bg.x), clamp01(bg.y), clamp01(bg.z));
+        normal = mk3(0, 0, 0);
+        return;
+    }
+    const DMaterial m = S.materials[h.mat];
+    normal = h.n;
+    if (m.type == MAT_METAL) {
+        albedo = mk3(m.albedo[0], m.albedo[1], m.albedo[2]);
+    } else if (m.type == MAT_DIELECTRIC) {
+        albedo = mk3(1, 1, 1);
+    } else {
+        const F3 t = tex_value(S, m.tex, h.u, h.v, h.p);
+        albedo = m.type == MAT_LIGHT ? mk3(clamp01(t.x), clamp01(t.y), clamp01(t.z)) : mk3(t.x, t.y, t.z);
+        if (m.type == MAT_ISOTROPIC) normal = mk3(0, 0, 0);
+    }
+}
+
 } // namespace rtb

@@ -147,6 +147,24 @@ struct AdaptiveBuffers {
     }
 };
 
+// Working set of rt_render_denoised / rt_render_aov, kept between calls like AdaptiveBuffers: the feature sums, the filter's ping-pong
+// colour and variance buffers, the blurred variance, the feature means and the filtered image.  The half accumulators are AdaptiveBuffers'.
+struct DenoiseBuffers {
+    int64_t* d_albedo = nullptr;
+    int64_t* d_normal = nullptr;
+    double* d_c[2] = {nullptr, nullptr};
+    double* d_v[2] = {nullptr, nullptr};
+    double* d_vbar = nullptr;
+    double* d_feat = nullptr;
+    double* d_linear = nullptr;
+    size_t cap = 0; // pixels (W * H)
+    void release() {
+        void* all[] = {d_albedo, d_normal, d_c[0], d_c[1], d_v[0], d_v[1], d_vbar, d_feat, d_linear};
+        for (void* p : all) if (p) cudaFree(p);
+        d_albedo = d_normal = nullptr; d_c[0] = d_c[1] = d_v[0] = d_v[1] = nullptr; d_vbar = d_feat = d_linear = nullptr; cap = 0;
+    }
+};
+
 // The committed scene on one more GPU (rt_render_multi): same flattened bytes, pointers re-based into this GPU's arena.
 struct Replica {
     int device = -1;
@@ -199,12 +217,14 @@ struct rt_scene {
     Workspace* workspace = nullptr;
     RenderBuffers out;
     AdaptiveBuffers adaptive;
+    DenoiseBuffers denoise;
     std::vector<Replica> replicas; // GPUs 1 .. n-1 of rt_render_multi (GPU 0 is `dev`)
     std::shared_ptr<void> debug_flat; // rt_debug_host_scene: the host-flattened arrays handed to the caller
     ~rt_scene() {
         for (Replica& r : replicas) r.release();
         out.release();
         adaptive.release();
+        denoise.release();
         dev.release();
         free_workspace(workspace);
     }
@@ -1899,6 +1919,148 @@ int32_t rt_render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_ad
 int32_t rt_render_adaptive_multi(rt_scene* s, const rt_render_config* cfg, const rt_adaptive_config* ac, int32_t n_gpus, double* out_screen,
                                  int64_t* out_accum, int32_t* out_samples, rt_stats* stats) {
     return render_adaptive(s, cfg, ac, n_gpus, out_screen, out_accum, out_samples, stats);
+}
+
+// ---- denoised renders (include/rtb200.h rt_render_aov / rt_render_denoised; the numpy reference is ray_tracing_series_rust_b200/denoise.py)
+namespace {
+
+int32_t ensure_denoise_buffers(rt_scene* s, size_t npix) {
+    DenoiseBuffers& b = s->denoise;
+    if (npix <= b.cap) return RT_OK;
+    b.release();
+    cudaError_t e;
+    const size_t n3 = npix * 3;
+    if ((e = cudaMalloc(&b.d_albedo, n3 * sizeof(int64_t))) != cudaSuccess || (e = cudaMalloc(&b.d_normal, n3 * sizeof(int64_t))) != cudaSuccess ||
+        (e = cudaMalloc(&b.d_c[0], n3 * sizeof(double))) != cudaSuccess || (e = cudaMalloc(&b.d_c[1], n3 * sizeof(double))) != cudaSuccess ||
+        (e = cudaMalloc(&b.d_v[0], npix * sizeof(double))) != cudaSuccess || (e = cudaMalloc(&b.d_v[1], npix * sizeof(double))) != cudaSuccess ||
+        (e = cudaMalloc(&b.d_vbar, npix * sizeof(double))) != cudaSuccess || (e = cudaMalloc(&b.d_feat, 2 * n3 * sizeof(double))) != cudaSuccess ||
+        (e = cudaMalloc(&b.d_linear, n3 * sizeof(double))) != cudaSuccess) {
+        b.release();
+        return fail_cuda(e, "denoise buffers");
+    }
+    b.cap = npix;
+    return RT_OK;
+}
+
+// the feature pass of job (its sample range) into the scene's zeroed feature sums; paths = segments = rays traced
+int32_t aov_pass(rt_scene* s, const RenderJob& job, cudaStream_t stream, rt_stats* st) {
+    DenoiseBuffers& b = s->denoise;
+    const size_t n = (size_t)job.width * job.height * 3;
+    cudaError_t e;
+    if ((e = cudaMemsetAsync(b.d_albedo, 0, n * sizeof(int64_t), stream)) != cudaSuccess || (e = cudaMemsetAsync(b.d_normal, 0, n * sizeof(int64_t), stream)) != cudaSuccess)
+        return fail_cuda(e, "feature set-up");
+    if ((e = launch_aov(s->dev.scene, job, b.d_albedo, b.d_normal, stream)) != cudaSuccess) return fail_cuda(e, "feature pass");
+    if (st) {
+        st->paths = st->segments = (uint64_t)job.width * (uint64_t)job.rows * (uint64_t)(job.sample_end - job.sample_begin);
+        st->kernel_launches = 1;
+    }
+    return RT_OK;
+}
+
+} // namespace
+
+int32_t RTB_FN(render_aov)(rt_scene* s, const rt_render_config* cfg, int64_t* out_albedo, int64_t* out_normal, rt_stats* stats) {
+    CHECK_SCENE(s);
+    if (!cfg) return fail(RT_ERR_INVALID, "null config");
+    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
+        return fail(RT_ERR_INVALID, "rt_render_aov takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
+    RenderJob job;
+    int32_t rc = make_job(s, cfg, job);
+    if (rc != RT_OK) return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    DeviceGuard guard(s->dev.device);
+    const size_t npix = (size_t)job.width * job.height, n = npix * 3;
+    if ((rc = ensure_out_buffers(s, n)) != RT_OK) return rc;
+    if ((rc = ensure_denoise_buffers(s, npix)) != RT_OK) return rc;
+    RenderBuffers& o = s->out;
+    rt_stats st;
+    std::memset(&st, 0, sizeof st);
+    if ((rc = aov_pass(s, job, o.stream, &st)) != RT_OK) return rc;
+    cudaError_t e;
+    if (out_albedo && (e = cudaMemcpyAsync(out_albedo, s->denoise.d_albedo, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "albedo copy");
+    if (out_normal && (e = cudaMemcpyAsync(out_normal, s->denoise.d_normal, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "normal copy");
+    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "feature sync");
+    if (stats) {
+        *stats = st;
+        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    return RT_OK;
+}
+
+int32_t rt_render_denoised(rt_scene* s, const rt_render_config* cfg, const rt_denoise_config* dc, double* out_screen, double* out_linear,
+                           int64_t* out_accum, rt_stats* stats) {
+    CHECK_SCENE(s);
+    if (!cfg) return fail(RT_ERR_INVALID, "null config");
+    // argument checks first: they need no committed scene
+    if (!dc) return fail(RT_ERR_INVALID, "null denoise config");
+    const int32_t n = cfg->samples_per_pixel;
+    if (n < 2) return fail(RT_ERR_INVALID, "rt_render_denoised needs samples_per_pixel >= 2 (two half renders)");
+    if (dc->aov_samples < 1 || dc->aov_samples > n) return fail(RT_ERR_INVALID, "denoise aov_samples outside 1..samples_per_pixel");
+    if (dc->iterations < 1 || dc->iterations > 8) return fail(RT_ERR_INVALID, "denoise iterations outside 1..8");
+    for (double sg : {dc->sigma_color, dc->sigma_albedo, dc->sigma_normal})
+        if (!(sg > 0.0) || !std::isfinite(sg)) return fail(RT_ERR_INVALID, "denoise sigmas must be finite and > 0");
+    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
+        return fail(RT_ERR_INVALID, "rt_render_denoised takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
+    if (cfg->sample_begin != 0 || (cfg->sample_end != 0 && cfg->sample_end != n))
+        return fail(RT_ERR_INVALID, "rt_render_denoised renders every sample range itself: sample_begin / sample_end must cover [0, samples_per_pixel)");
+    RenderJob job;
+    int32_t rc = make_job(s, cfg, job);
+    if (rc != RT_OK) return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    DeviceGuard guard(s->dev.device);
+    const size_t npix = (size_t)job.width * job.height, n3 = npix * 3;
+    if ((rc = ensure_out_buffers(s, n3)) != RT_OK) return rc;
+    if ((rc = ensure_adaptive_buffers(s, npix)) != RT_OK) return rc;
+    if ((rc = ensure_denoise_buffers(s, npix)) != RT_OK) return rc;
+    RenderBuffers& o = s->out;
+    AdaptiveBuffers& ab = s->adaptive;
+    DenoiseBuffers& db = s->denoise;
+    const RenderTuning tune = tuning_for(s, cfg);
+    const int32_t hA = n / 2;
+    cudaError_t e;
+    if ((e = cudaMemsetAsync(ab.d_a, 0, n3 * sizeof(int64_t), o.stream)) != cudaSuccess || (e = cudaMemsetAsync(ab.d_b, 0, n3 * sizeof(int64_t), o.stream)) != cudaSuccess)
+        return fail_cuda(e, "denoise set-up");
+    rt_stats sum;
+    std::memset(&sum, 0, sizeof sum);
+    // the two half renders: samples [0, hA) into A and [hA, n) into B (their sum is rt_render's accumulator bit for bit)
+    for (int half = 0; half < 2; ++half) {
+        RenderJob hj = job;
+        hj.sample_begin = half ? hA : 0;
+        hj.sample_end = half ? n : hA;
+        rt_stats rs;
+        std::memset(&rs, 0, sizeof rs);
+        if ((e = launch_render(s->dev.scene, hj, tune, half ? ab.d_b : ab.d_a, o.stream, &rs, &s->workspace)) != cudaSuccess) return fail_cuda(e, "denoise half render");
+        add_stats(sum, rs, false);
+    }
+    RenderJob aj = job;
+    aj.sample_begin = 0;
+    aj.sample_end = dc->aov_samples;
+    rt_stats as;
+    std::memset(&as, 0, sizeof as);
+    if ((rc = aov_pass(s, aj, o.stream, &as)) != RT_OK) return rc;
+    sum.kernel_launches += as.kernel_launches;
+    DenoiseJob dj;
+    dj.a = ab.d_a; dj.b = ab.d_b; dj.albedo = db.d_albedo; dj.normal = db.d_normal;
+    dj.W = job.width; dj.H = job.height; dj.rows = job.rows; dj.hA = hA; dj.hB = n - hA; dj.m = dc->aov_samples; dj.iterations = dc->iterations;
+    dj.sigma_color = dc->sigma_color; dj.sigma_albedo = dc->sigma_albedo; dj.sigma_normal = dc->sigma_normal;
+    dj.c[0] = db.d_c[0]; dj.c[1] = db.d_c[1]; dj.v[0] = db.d_v[0]; dj.v[1] = db.d_v[1]; dj.vbar = db.d_vbar; dj.feat = db.d_feat;
+    dj.accum_out = o.d_accum; dj.linear_out = db.d_linear; dj.screen_u8 = o.d_u8;
+    if ((e = launch_denoise(dj, o.stream)) != cudaSuccess) return fail_cuda(e, "denoise filter");
+    sum.kernel_launches += 2 + 2 * (uint64_t)dc->iterations;
+    if (out_screen && (e = cudaMemcpyAsync(o.h_u8, o.d_u8, n3, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "screen copy");
+    if (out_linear && (e = cudaMemcpyAsync(out_linear, db.d_linear, n3 * sizeof(double), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "linear copy");
+    if (out_accum && (e = cudaMemcpyAsync(out_accum, o.d_accum, n3 * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "accum copy");
+    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "denoise sync");
+    if (out_screen) widen_screen(o.h_u8, out_screen, n3);
+    if (stats) {
+        *stats = sum;
+        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    return RT_OK;
 }
 
 // ---- peer group: the exchange of the one-process-per-GPU layout without a collective library on the data path
