@@ -120,12 +120,15 @@ struct RenderBuffers {
     }
 };
 
-// Working set of rt_render_adaptive, kept between calls like RenderBuffers: the half accumulators A and B, the active pixel list and
+// Half accumulators A | B in one block, GPU 0's and a replica's alike: B starts half_offset(n) elements after A, an even offset that
+// keeps B 16-byte aligned for the kernels' 128-bit loads when n is odd.
+size_t half_offset(size_t n) { return (n + 1) & ~(size_t)1; }
+
+// Working set of rt_render_adaptive, kept between calls like RenderBuffers: the half accumulators A | B, the active pixel list and
 // the next one, per-pixel sample counts, the convergence mask, the compaction flags and CUB's temp storage; the pinned count word the
 // host reads once per check point.
 struct AdaptiveBuffers {
-    int64_t* d_a = nullptr;
-    int64_t* d_b = nullptr;
+    int64_t* d_ab = nullptr;
     uint32_t* d_list[2] = {nullptr, nullptr};
     int32_t* d_samples = nullptr;
     uint8_t* d_u = nullptr;
@@ -135,15 +138,14 @@ struct AdaptiveBuffers {
     uint32_t* h_count = nullptr; // pinned
     size_t cap = 0;              // pixels (W * H)
     void release() {
-        if (d_a) cudaFree(d_a);
-        if (d_b) cudaFree(d_b);
+        if (d_ab) cudaFree(d_ab);
         for (uint32_t*& l : d_list) { if (l) cudaFree(l); l = nullptr; }
         if (d_samples) cudaFree(d_samples);
         if (d_u) cudaFree(d_u);
         if (d_keep) cudaFree(d_keep);
         if (d_temp) cudaFree(d_temp);
         if (h_count) cudaFreeHost(h_count);
-        d_a = d_b = nullptr; d_samples = nullptr; d_u = d_keep = nullptr; d_temp = nullptr; temp_bytes = 0; h_count = nullptr; cap = 0;
+        d_ab = nullptr; d_samples = nullptr; d_u = d_keep = nullptr; d_temp = nullptr; temp_bytes = 0; h_count = nullptr; cap = 0;
     }
 };
 
@@ -165,6 +167,16 @@ struct DenoiseBuffers {
     }
 };
 
+// grow-only buffer on the current device: reallocated to need + headroom elements (contents dropped) when it holds fewer than need
+template <class T> cudaError_t grow(T*& p, size_t& cap, size_t need, size_t headroom = 0) {
+    if (need <= cap) return cudaSuccess;
+    if (p) cudaFree(p);
+    p = nullptr; cap = 0;
+    const cudaError_t e = cudaMalloc(&p, (need + headroom) * sizeof(T));
+    if (e == cudaSuccess) cap = need + headroom;
+    return e;
+}
+
 // The committed scene on one more GPU (rt_render_multi): same flattened bytes, pointers re-based into this GPU's arena.
 struct Replica {
     int device = -1;
@@ -173,7 +185,7 @@ struct Replica {
     uint64_t generation = ~0ull;
     DeviceScene scene;
     Workspace* workspace = nullptr;
-    int64_t* d_accum = nullptr; // rt_render_multi's shard; rt_render_adaptive_multi's half accumulators A | B (B at an even offset)
+    int64_t* d_accum = nullptr; // rt_render_multi's shard; rt_render_adaptive_multi's half accumulators A | B (B at half_offset)
     size_t accum_cap = 0;
     uint32_t* d_list = nullptr; // rt_render_adaptive_multi: this GPU's copy of the active pixel list
     size_t list_cap = 0;
@@ -287,6 +299,23 @@ template <class F> void parallel_chunks(size_t n, F&& body) {
     }
     body((size_t)0, std::min(n, chunk));
     for (std::thread& th : pool) th.join();
+}
+
+// body(g) for every GPU g < n at the same time: GPUs 1..n-1 on threads of their own, GPU 0 on the calling thread; every thread
+// started is joined.  If a thread cannot be started, GPU 0's body does not run: on_start_failure() must let the started ones finish.
+template <class Body, class OnStartFailure> int32_t run_on_gpus(int n, Body&& body, OnStartFailure&& on_start_failure) {
+    std::vector<std::thread> pool;
+    try {
+        pool.reserve((size_t)n - 1);
+        for (int g = 1; g < n; ++g) pool.emplace_back([&body, g] { body(g); });
+    } catch (const std::exception&) {
+        on_start_failure();
+        for (std::thread& th : pool) th.join();
+        return fail(RT_ERR_CUDA, "could not start the render threads");
+    }
+    body(0);
+    for (std::thread& th : pool) th.join();
+    return RT_OK;
 }
 
 struct FlatPrim {
@@ -1355,19 +1384,8 @@ static RenderTuning tuning_for_flags(const rt_scene* s, const rt_render_config* 
 }
 
 int32_t rt_render_device(rt_scene* s, const rt_render_config* cfg, int64_t* d_accum, void* cuda_stream, rt_stats* stats) {
-    CHECK_SCENE(s);
-    if (!d_accum) return fail(RT_ERR_INVALID, "null accumulator");
-    RenderJob job;
-    const int32_t r = make_job(s, cfg, job);
-    if (r != RT_OK) return r;
-    if (stats) std::memset(stats, 0, sizeof *stats);
-    const auto t0 = std::chrono::steady_clock::now();
-    RenderTuning tune = tuning_for_flags(s, cfg);
-    tune.no_wait = (cfg->flags & RT_RENDER_NO_WAIT) ? 1 : 0;
-    const cudaError_t e = launch_render(s->dev.scene, job, tune, d_accum, (cudaStream_t)cuda_stream, stats, &s->workspace);
-    if (e != cudaSuccess) return fail_cuda(e, "render");
-    if (stats) stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    return RT_OK;
+    // every path: launch_render clamps the range to the job's own paths
+    return rt_render_device_paths(s, cfg, 0, UINT64_MAX, d_accum, cuda_stream, stats);
 }
 
 int32_t rt_render_device_paths(rt_scene* s, const rt_render_config* cfg, uint64_t path_begin, uint64_t path_end, int64_t* d_accum, void* cuda_stream, rt_stats* stats) {
@@ -1377,12 +1395,9 @@ int32_t rt_render_device_paths(rt_scene* s, const rt_render_config* cfg, uint64_
     const int32_t r = make_job(s, cfg, job);
     if (r != RT_OK) return r;
     if (path_begin > path_end) return fail(RT_ERR_INVALID, "bad path range");
-    if (path_begin == path_end) { // an empty shard renders nothing
-        if (stats) std::memset(stats, 0, sizeof *stats);
-        return RT_OK;
-    }
-    job.path_begin = path_begin; job.path_end = path_end;
     if (stats) std::memset(stats, 0, sizeof *stats);
+    if (path_begin == path_end) return RT_OK; // an empty shard renders nothing
+    job.path_begin = path_begin; job.path_end = path_end;
     const auto t0 = std::chrono::steady_clock::now();
     RenderTuning tune = tuning_for_flags(s, cfg);
     tune.no_wait = (cfg->flags & RT_RENDER_NO_WAIT) ? 1 : 0;
@@ -1401,20 +1416,6 @@ int32_t rt_resolve_device(const int64_t* d_accum, double* d_screen, int32_t widt
 
 // ---- rt_render / rt_render_multi: host-buffer entry points (what a Rust render_scene_gpu calls, world.rs:1181-1247)
 namespace {
-
-// The host-buffer entry points run on the device the scene was committed on, whatever device is current in the calling thread, and
-// leave the caller's current device as they found it.
-struct DeviceGuard {
-    int home = -1;
-    explicit DeviceGuard(int dev) {
-        if (cudaGetDevice(&home) != cudaSuccess) home = -1;
-        if (home != dev) cudaSetDevice(dev);
-    }
-    ~DeviceGuard() {
-        int cur = -1;
-        if (home >= 0 && cudaGetDevice(&cur) == cudaSuccess && cur != home) cudaSetDevice(home);
-    }
-};
 
 int32_t ensure_out_buffers(rt_scene* s, size_t n) {
     RenderBuffers& o = s->out;
@@ -1437,48 +1438,71 @@ void widen_screen(const uint8_t* src, double* dst, size_t n) {
     for (size_t i = 0; i < n; ++i) dst[i] = (double)src[i];
 }
 
-// sum of the shards (own + peers) -> out buffers on the gathering GPU -> host
-int32_t gather_and_copy_out(rt_scene* s, const AccumShards& shards, const RenderJob& job, double* out_screen, int64_t* out_accum) {
-    RenderBuffers& o = s->out;
-    const size_t n = (size_t)job.width * job.height * 3;
-    cudaError_t e;
-    // one shard: its sums already are o.d_accum; several: summed in place over shard 0 (a thread reads element i of every shard before it writes it)
-    int64_t* sum_out = (out_accum && shards.n > 1) ? o.d_accum : nullptr;
-    if ((e = launch_reduce_resolve(shards, sum_out, out_screen ? o.d_u8 : nullptr, nullptr, job.width, job.height, job.spp_total, job.rows, o.stream)) != cudaSuccess)
-        return fail_cuda(e, "reduce + resolve");
-    if (out_screen && (e = cudaMemcpyAsync(o.h_u8, o.d_u8, n, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "screen copy");
-    if (out_accum && (e = cudaMemcpyAsync(out_accum, o.d_accum, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "accum copy");
-    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "render sync");
-    if (out_screen) widen_screen(o.h_u8, out_screen, n);
+// a device-to-host copy at the end of a host-buffer render; skipped when dst is null
+struct Download {
+    void* dst;
+    const void* src;
+    size_t bytes;
+    const char* what;
+};
+
+// One host-buffer render call.  begin() runs after the entry point's own argument checks (they need no committed scene): make_job,
+// then the output buffers on the device the scene was committed on.  That device stays current until the call returns, whatever
+// device was current in the calling thread, which gets its own back.  finish() is the copy-out the call ends with.
+struct HostRender {
+    rt_scene* s = nullptr;
+    RenderJob job;
+    size_t npix = 0, n = 0; // pixels; accumulator elements (npix * 3)
+    std::chrono::steady_clock::time_point t0;
+    int home = -1; // the calling thread's device
+
+    // shards_image: the call cuts the image over its GPUs itself, so a tile shard in cfg is refused
+    int32_t begin(rt_scene* scene, const rt_render_config* cfg, bool shards_image = false) {
+        s = scene;
+        const int32_t rc = make_job(s, cfg, job);
+        if (rc != RT_OK) return rc;
+        if (shards_image && job.tile_count > 1) return fail(RT_ERR_INVALID, "rt_render_multi shards the image itself: RT_RENDER_TILE_SHARD must not be set");
+        t0 = std::chrono::steady_clock::now();
+        if (cudaGetDevice(&home) != cudaSuccess) home = -1;
+        if (home != s->dev.device) cudaSetDevice(s->dev.device);
+        npix = (size_t)job.width * job.height;
+        n = npix * 3;
+        return ensure_out_buffers(s, n);
+    }
+    ~HostRender() {
+        int cur = -1;
+        if (home >= 0 && cudaGetDevice(&cur) == cudaSuccess && cur != home) cudaSetDevice(home);
+    }
+
+    // On the scene's stream: the byte Screen's copy (when out_screen) and the downloads in order, one sync, the Screen widened to
+    // f64; then stats = sum with the call's ms_total.
+    int32_t finish(double* out_screen, std::initializer_list<Download> downloads, const char* sync_what, const rt_stats& sum, rt_stats* stats) const {
+        RenderBuffers& o = s->out;
+        cudaError_t e;
+        if (out_screen && (e = cudaMemcpyAsync(o.h_u8, o.d_u8, n, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "screen copy");
+        for (const Download& d : downloads)
+            if (d.dst && (e = cudaMemcpyAsync(d.dst, d.src, d.bytes, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, d.what);
+        if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, sync_what);
+        if (out_screen) widen_screen(o.h_u8, out_screen, n);
+        if (stats) {
+            *stats = sum;
+            stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        }
+        return RT_OK;
+    }
+};
+
+// The entry points that render the whole image themselves take neither a tile shard nor RT_RENDER_NO_WAIT; all_samples: nor a
+// sample range other than [0, samples_per_pixel).
+int32_t check_whole_render(const rt_render_config* cfg, const char* name, bool all_samples) {
+    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
+        return fail(RT_ERR_INVALID, std::string(name) + " takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
+    if (all_samples && (cfg->sample_begin != 0 || (cfg->sample_end != 0 && cfg->sample_end != cfg->samples_per_pixel)))
+        return fail(RT_ERR_INVALID, std::string(name) + " renders every sample range itself: sample_begin / sample_end must cover [0, samples_per_pixel)");
     return RT_OK;
 }
-
-RenderTuning tuning_for(const rt_scene* s, const rt_render_config* cfg) { return tuning_for_flags(s, cfg); }
 
 } // namespace
-
-int32_t rt_render(rt_scene* s, const rt_render_config* cfg, double* out_screen, int64_t* out_accum, rt_stats* stats) {
-    CHECK_SCENE(s);
-    RenderJob job;
-    int32_t rc = make_job(s, cfg, job);
-    if (rc != RT_OK) return rc;
-    const auto t0 = std::chrono::steady_clock::now();
-    DeviceGuard guard(s->dev.device);
-    const size_t n = (size_t)job.width * job.height * 3;
-    if ((rc = ensure_out_buffers(s, n)) != RT_OK) return rc;
-    RenderBuffers& o = s->out;
-    cudaError_t e;
-    if ((e = cudaMemsetAsync(o.d_accum, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess) return fail_cuda(e, "memset");
-    if (stats) std::memset(stats, 0, sizeof *stats);
-    if ((e = launch_render(s->dev.scene, job, tuning_for(s, cfg), o.d_accum, o.stream, stats, &s->workspace)) != cudaSuccess) return fail_cuda(e, "render");
-    AccumShards sh;
-    std::memset(&sh, 0, sizeof sh);
-    sh.n = 1;
-    sh.p[0] = o.d_accum;
-    if ((rc = gather_and_copy_out(s, sh, job, out_screen, out_accum)) != RT_OK) return rc;
-    if (stats) stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    return RT_OK;
-}
 
 // ---- adaptive sampling (include/rtb200.h rt_render_adaptive; the numpy mirror is ray_tracing_series_rust_b200/adaptive.py)
 namespace {
@@ -1489,7 +1513,7 @@ int32_t ensure_adaptive_buffers(rt_scene* s, size_t npix) {
     b.release();
     cudaError_t e;
     const size_t temp = adaptive_select_temp_bytes((uint32_t)npix);
-    if ((e = cudaMalloc(&b.d_a, npix * 3 * sizeof(int64_t))) != cudaSuccess || (e = cudaMalloc(&b.d_b, npix * 3 * sizeof(int64_t))) != cudaSuccess ||
+    if ((e = cudaMalloc(&b.d_ab, 2 * half_offset(npix * 3) * sizeof(int64_t))) != cudaSuccess ||
         (e = cudaMalloc(&b.d_list[0], npix * sizeof(uint32_t))) != cudaSuccess || (e = cudaMalloc(&b.d_list[1], npix * sizeof(uint32_t))) != cudaSuccess ||
         (e = cudaMalloc(&b.d_samples, npix * sizeof(int32_t))) != cudaSuccess || (e = cudaMalloc(&b.d_u, npix)) != cudaSuccess ||
         (e = cudaMalloc(&b.d_keep, npix)) != cudaSuccess || (e = cudaMalloc(&b.d_temp, std::max<size_t>(temp, 1))) != cudaSuccess ||
@@ -1536,7 +1560,9 @@ bool multi_alias() { // test hook: every logical GPU is the scene's own device (
 // logical GPU g (>= 1) -> physical device: the devices after the scene's own, wrapping around
 int32_t replica_device(const rt_scene* s, int g, int dev_count) { return multi_alias() ? s->dev.device : (s->dev.device + g) % dev_count; }
 
-int32_t ensure_replicas(rt_scene* s, int32_t n_gpus, size_t accum_elems) {
+// GPUs 1 .. n_gpus-1: the committed scene, a stream, an accumulator block of accum_elems (and as large a staging block next to GPU 0
+// when GPU 0 cannot read it in place), a pixel list of list_elems
+int32_t ensure_replicas(rt_scene* s, int32_t n_gpus, size_t accum_elems, size_t list_elems) {
     int dev_count = 0;
     cudaError_t e = cudaGetDeviceCount(&dev_count);
     if (e != cudaSuccess || dev_count < 1) return fail(RT_ERR_CUDA, "no CUDA device: librtb200 has no CPU fallback");
@@ -1553,22 +1579,12 @@ int32_t ensure_replicas(rt_scene* s, int32_t n_gpus, size_t accum_elems) {
         if ((e = cudaSetDevice(dev)) != cudaSuccess) { rc = fail_cuda(e, "cudaSetDevice"); break; }
         if (!r.stream && (e = cudaStreamCreateWithFlags(&r.stream, cudaStreamNonBlocking)) != cudaSuccess) { rc = fail_cuda(e, "replica stream"); break; }
         if (r.generation != s->dev.generation) { // upload the committed bytes (still in the pinned staging buffer) to this GPU
-            if (s->dev.bytes > r.capacity) {
-                if (r.arena) cudaFree(r.arena);
-                r.arena = nullptr; r.capacity = 0;
-                const size_t cap = s->dev.bytes + s->dev.bytes / 4 + 4096;
-                if ((e = cudaMalloc(&r.arena, cap)) != cudaSuccess) { rc = fail_cuda(e, "replica arena"); break; }
-                r.capacity = cap;
-            }
+            if ((e = grow(r.arena, r.capacity, s->dev.bytes, s->dev.bytes / 4 + 4096)) != cudaSuccess) { rc = fail_cuda(e, "replica arena"); break; }
             if ((e = cudaMemcpyAsync(r.arena, s->dev.staging, s->dev.bytes, cudaMemcpyHostToDevice, r.stream)) != cudaSuccess) { rc = fail_cuda(e, "replica upload"); break; }
             r.generation = s->dev.generation;
         }
-        if (accum_elems > r.accum_cap) {
-            if (r.d_accum) cudaFree(r.d_accum);
-            r.d_accum = nullptr; r.accum_cap = 0;
-            if ((e = cudaMalloc(&r.d_accum, accum_elems * sizeof(int64_t))) != cudaSuccess) { rc = fail_cuda(e, "replica accumulator"); break; }
-            r.accum_cap = accum_elems;
-        }
+        if ((e = grow(r.d_accum, r.accum_cap, accum_elems)) != cudaSuccess) { rc = fail_cuda(e, "replica accumulator"); break; }
+        if ((e = grow(r.d_list, r.list_cap, list_elems)) != cudaSuccess) { rc = fail_cuda(e, "replica pixel list"); break; }
         // scalars (camera, background, flags) follow the primary scene; pointers are re-based into this arena
         r.scene = s->dev.scene;
         for (const auto& fo : s->dev.layout) {
@@ -1586,12 +1602,9 @@ int32_t ensure_replicas(rt_scene* s, int32_t n_gpus, size_t accum_elems) {
                 if (e == cudaSuccess || e == cudaErrorPeerAccessAlreadyEnabled) r.peer_ok = true;
                 (void)cudaGetLastError();
             }
-            if (!r.peer_ok && accum_elems > r.stage_cap) { // no P2P route: the shard is copied next to the gathering GPU's own first
+            if (!r.peer_ok) { // no P2P route: the shard is copied next to the gathering GPU's own first
                 cudaSetDevice(s->dev.device);
-                if (r.d_stage) cudaFree(r.d_stage);
-                r.d_stage = nullptr; r.stage_cap = 0;
-                if ((e = cudaMalloc(&r.d_stage, accum_elems * sizeof(int64_t))) != cudaSuccess) { rc = fail_cuda(e, "gather staging"); break; }
-                r.stage_cap = accum_elems;
+                if ((e = grow(r.d_stage, r.stage_cap, accum_elems)) != cudaSuccess) { rc = fail_cuda(e, "gather staging"); break; }
             }
         }
     }
@@ -1599,93 +1612,110 @@ int32_t ensure_replicas(rt_scene* s, int32_t n_gpus, size_t accum_elems) {
     return rc;
 }
 
+// GPU g of a render over several, as its render thread uses it: g = 0 is the scene's own device, scene, stream and workspace, g >= 1
+// replica g - 1.  accum: the GPU's accumulator block (rt_render_multi's shard, the adaptive A | B); GPU 0's is accum0.
+struct GpuView {
+    int device;
+    const DeviceScene* scene;
+    cudaStream_t stream;
+    Workspace** workspace;
+    int64_t* accum;
+};
+
+GpuView gpu_view(rt_scene* s, int g, int64_t* accum0) {
+    if (g == 0) return {s->dev.device, &s->dev.scene, s->out.stream, &s->workspace, accum0};
+    Replica& r = s->replicas[(size_t)g - 1];
+    return {r.device, &r.scene, r.stream, &r.workspace, r.d_accum};
+}
+
+// Every GPU's accumulator block of elems elements as GPU 0 reads it, into p[g]: GPU 0's own (own) and each replica's in place where GPU 0
+// can address it (P2P-mapped, or alias mode), otherwise copied into the replica's staging block next to GPU 0 on GPU 0's stream.
+cudaError_t gather_blocks(rt_scene* s, int n_gpus, const int64_t* own, size_t elems, const int64_t** p) {
+    p[0] = own;
+    for (int g = 1; g < n_gpus; ++g) {
+        Replica& r = s->replicas[(size_t)g - 1];
+        p[g] = r.d_accum;
+        if (r.peer_ok) continue;
+        const cudaError_t e = cudaMemcpyPeerAsync(r.d_stage, s->dev.device, r.d_accum, r.device, elems * sizeof(int64_t), s->out.stream);
+        if (e != cudaSuccess) return e;
+        p[g] = r.d_stage;
+    }
+    return cudaSuccess;
+}
+
+// rt_render (n_gpus = 1: the job is not split) and rt_render_multi: GPU g renders shard g into its own accumulator, then GPU 0 sums
+// the shards and resolves them in one kernel.
+int32_t render_shards(rt_scene* s, const rt_render_config* cfg, int32_t n_gpus, int32_t shard_mode, double* out_screen, int64_t* out_accum,
+                      rt_stats* stats) {
+    HostRender call;
+    int32_t rc = call.begin(s, cfg, n_gpus > 1);
+    if (rc != RT_OK) return rc;
+    const RenderJob& job = call.job;
+    const size_t n = call.n;
+    if (n_gpus > 1 && (rc = ensure_replicas(s, n_gpus, n, 0)) != RT_OK) return rc;
+    RenderBuffers& o = s->out;
+    const RenderTuning tune = tuning_for_flags(s, cfg);
+    rt_stats st[RT_MAX_GPUS] = {};
+    cudaError_t errs[RT_MAX_GPUS] = {};
+    const char* what[RT_MAX_GPUS] = {};
+    auto run = [&](int g) {
+        // shard g: the g-th of N equal ranges of the paths (sample-major: sample ranges of every pixel, cut evenly), or every sample of the 4-row bands b with b % N == g
+        RenderJob sj = job;
+        if (n_gpus > 1 && shard_mode == RT_SHARD_SAMPLES) { // an even share of the paths in sample-major order: whole samples plus a partial first / last one
+            const uint64_t T = (uint64_t)job.width * (uint64_t)job.rows * (uint64_t)(job.sample_end - job.sample_begin);
+            sj.path_begin = T * (uint64_t)g / (uint64_t)n_gpus;
+            sj.path_end = T * (uint64_t)(g + 1) / (uint64_t)n_gpus;
+            if (sj.path_end == sj.path_begin) sj.sample_end = sj.sample_begin; // nothing for this GPU
+        } else if (n_gpus > 1) {
+            sj.tile_rank = g;
+            sj.tile_count = n_gpus;
+        }
+        const GpuView v = gpu_view(s, g, o.d_accum);
+        cudaError_t& e = errs[g];
+        what[g] = "memset";
+        if ((g == 0 || (e = cudaSetDevice(v.device)) == cudaSuccess) && (e = cudaMemsetAsync(v.accum, 0, n * sizeof(int64_t), v.stream)) == cudaSuccess) {
+            what[g] = "render";
+            e = launch_render(*v.scene, sj, tune, v.accum, v.stream, &st[g], v.workspace); // returns after its stream has drained
+        }
+    };
+    if ((rc = run_on_gpus(n_gpus, run, [] {})) != RT_OK) return rc;
+    for (int g = 0; g < n_gpus; ++g)
+        if (errs[g] != cudaSuccess) return fail_cuda(errs[g], n_gpus > 1 ? "render (multi-GPU shard)" : what[g]);
+    AccumShards sh;
+    std::memset(&sh, 0, sizeof sh);
+    sh.n = n_gpus;
+    cudaError_t e;
+    if ((e = gather_blocks(s, n_gpus, o.d_accum, n, sh.p)) != cudaSuccess) return fail_cuda(e, "peer copy");
+    // one shard: its sums already are o.d_accum; several: summed in place over shard 0 (a thread reads element i of every shard before it writes it)
+    int64_t* sum_out = (out_accum && n_gpus > 1) ? o.d_accum : nullptr;
+    if ((e = launch_reduce_resolve(sh, sum_out, out_screen ? o.d_u8 : nullptr, nullptr, job.width, job.height, job.spp_total, job.rows, o.stream)) != cudaSuccess)
+        return fail_cuda(e, "reduce + resolve");
+    rt_stats sum = st[0];
+    for (int g = 1; g < n_gpus; ++g) add_stats(sum, st[g], true); // ms_device: the slowest shard
+    if (n_gpus > 1) sum.kernel_launches += 1;                       // k_reduce_resolve
+    return call.finish(out_screen, {{out_accum, o.d_accum, n * sizeof(int64_t), "accum copy"}}, "render sync", sum, stats);
+}
+
 } // namespace
+
+int32_t rt_render(rt_scene* s, const rt_render_config* cfg, double* out_screen, int64_t* out_accum, rt_stats* stats) {
+    CHECK_SCENE(s);
+    return render_shards(s, cfg, 1, RT_SHARD_SAMPLES, out_screen, out_accum, stats);
+}
 
 int32_t rt_scene_commit_multi(rt_scene* s, int32_t n_gpus) {
     CHECK_SCENE(s);
     if (n_gpus < 1) return fail(RT_ERR_INVALID, "n_gpus < 1");
     const int32_t rc = do_commit(s);
     if (rc != RT_OK) return rc;
-    return ensure_replicas(s, n_gpus, 0);
+    return ensure_replicas(s, n_gpus, 0, 0);
 }
 
 int32_t rt_render_multi(rt_scene* s, const rt_render_config* cfg, int32_t n_gpus, int32_t shard_mode, double* out_screen, int64_t* out_accum, rt_stats* stats) {
     CHECK_SCENE(s);
     if (n_gpus < 1) return fail(RT_ERR_INVALID, "n_gpus < 1");
     if (shard_mode != RT_SHARD_SAMPLES && shard_mode != RT_SHARD_TILES) return fail(RT_ERR_INVALID, "shard_mode must be RT_SHARD_SAMPLES or RT_SHARD_TILES");
-    if (n_gpus == 1) return rt_render(s, cfg, out_screen, out_accum, stats);
-    RenderJob job;
-    int32_t rc = make_job(s, cfg, job);
-    if (rc != RT_OK) return rc;
-    if (job.tile_count > 1) return fail(RT_ERR_INVALID, "rt_render_multi shards the image itself: RT_RENDER_TILE_SHARD must not be set");
-    const auto t0 = std::chrono::steady_clock::now();
-    DeviceGuard guard(s->dev.device);
-    const size_t n = (size_t)job.width * job.height * 3;
-    if ((rc = ensure_out_buffers(s, n)) != RT_OK) return rc;
-    if ((rc = ensure_replicas(s, n_gpus, n)) != RT_OK) return rc;
-    const RenderTuning tune = tuning_for(s, cfg);
-    // shard g: the g-th of N equal ranges of the paths (sample-major: sample ranges of every pixel, cut evenly), or every sample of the 4-row bands b with b % N == g
-    std::vector<RenderJob> jobs((size_t)n_gpus, job);
-    const int32_t S = job.sample_end - job.sample_begin;
-    for (int g = 0; g < n_gpus; ++g) {
-        if (shard_mode == RT_SHARD_SAMPLES) { // an even share of the paths in sample-major order: whole samples plus a partial first / last one
-            const uint64_t T = (uint64_t)job.width * (uint64_t)job.rows * (uint64_t)S;
-            jobs[(size_t)g].path_begin = T * (uint64_t)g / (uint64_t)n_gpus;
-            jobs[(size_t)g].path_end = T * (uint64_t)(g + 1) / (uint64_t)n_gpus;
-            if (jobs[(size_t)g].path_end == jobs[(size_t)g].path_begin) jobs[(size_t)g].sample_end = jobs[(size_t)g].sample_begin; // nothing for this GPU
-        } else {
-            jobs[(size_t)g].tile_rank = g;
-            jobs[(size_t)g].tile_count = n_gpus;
-        }
-    }
-    std::vector<rt_stats> st((size_t)n_gpus);
-    std::vector<cudaError_t> errs((size_t)n_gpus, cudaSuccess);
-    auto run = [&](int g) {
-        rt_stats& out = st[(size_t)g];
-        std::memset(&out, 0, sizeof out);
-        cudaError_t e;
-        if (g == 0) {
-            RenderBuffers& o = s->out;
-            if ((e = cudaSetDevice(s->dev.device)) == cudaSuccess && (e = cudaMemsetAsync(o.d_accum, 0, n * sizeof(int64_t), o.stream)) == cudaSuccess)
-                e = launch_render(s->dev.scene, jobs[0], tune, o.d_accum, o.stream, &out, &s->workspace);
-        } else {
-            Replica& r = s->replicas[(size_t)g - 1];
-            if ((e = cudaSetDevice(r.device)) == cudaSuccess && (e = cudaMemsetAsync(r.d_accum, 0, n * sizeof(int64_t), r.stream)) == cudaSuccess)
-                e = launch_render(r.scene, jobs[(size_t)g], tune, r.d_accum, r.stream, &out, &r.workspace);
-        }
-        errs[(size_t)g] = e;
-    };
-    {
-        std::vector<std::thread> pool;
-        for (int g = 1; g < n_gpus; ++g) pool.emplace_back(run, g);
-        run(0); // launch_render returns after its stream has drained
-        for (std::thread& th : pool) th.join();
-    }
-    cudaSetDevice(s->dev.device);
-    for (int g = 0; g < n_gpus; ++g)
-        if (errs[(size_t)g] != cudaSuccess) return fail_cuda(errs[(size_t)g], "render (multi-GPU shard)");
-    AccumShards sh;
-    std::memset(&sh, 0, sizeof sh);
-    sh.n = n_gpus;
-    sh.p[0] = s->out.d_accum;
-    for (int g = 1; g < n_gpus; ++g) {
-        Replica& r = s->replicas[(size_t)g - 1];
-        if (r.peer_ok) {
-            sh.p[g] = r.d_accum;
-        } else {
-            const cudaError_t e = cudaMemcpyPeerAsync(r.d_stage, s->dev.device, r.d_accum, r.device, n * sizeof(int64_t), s->out.stream);
-            if (e != cudaSuccess) return fail_cuda(e, "peer copy");
-            sh.p[g] = r.d_stage;
-        }
-    }
-    if ((rc = gather_and_copy_out(s, sh, job, out_screen, out_accum)) != RT_OK) return rc;
-    if (stats) {
-        *stats = st[0];
-        for (int g = 1; g < n_gpus; ++g) add_stats(*stats, st[(size_t)g], true); // ms_device: the slowest shard
-        stats->kernel_launches += 1; // k_reduce_resolve
-        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    }
-    return RT_OK;
+    return render_shards(s, cfg, n_gpus, shard_mode, out_screen, out_accum, stats);
 }
 
 // ---- adaptive sampling on one GPU or several (rt_render_adaptive, rt_render_adaptive_multi)
@@ -1748,63 +1778,32 @@ int32_t render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adapt
     if (!(ac->threshold >= 0.0) || !std::isfinite(ac->threshold)) return fail(RT_ERR_INVALID, "adaptive threshold must be finite and >= 0");
     if (ac->radius < 0 || ac->radius > 8) return fail(RT_ERR_INVALID, "adaptive radius outside 0..8");
     if (ac->min_samples < 0 || ac->min_samples > cfg->samples_per_pixel) return fail(RT_ERR_INVALID, "adaptive min_samples outside 0..samples_per_pixel");
-    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
-        return fail(RT_ERR_INVALID, "rt_render_adaptive takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
-    if (cfg->sample_begin != 0 || (cfg->sample_end != 0 && cfg->sample_end != cfg->samples_per_pixel))
-        return fail(RT_ERR_INVALID, "rt_render_adaptive renders every sample range itself: sample_begin / sample_end must cover [0, samples_per_pixel)");
-    if (n_gpus < 1 || n_gpus > RT_MAX_GPUS) return fail(RT_ERR_INVALID, "n_gpus outside 1..16");
-    RenderJob job;
-    int32_t rc = make_job(s, cfg, job);
+    int32_t rc = check_whole_render(cfg, "rt_render_adaptive", true);
     if (rc != RT_OK) return rc;
-    const auto t0 = std::chrono::steady_clock::now();
-    DeviceGuard guard(s->dev.device);
-    const size_t npix = (size_t)job.width * job.height, n = npix * 3;
-    // A replica's B starts nb elements after its A: an even offset keeps B 16-byte aligned for the kernels' 128-bit loads when n is odd
-    const size_t nb = (n + 1) & ~(size_t)1;
-    if ((rc = ensure_out_buffers(s, n)) != RT_OK) return rc;
+    if (n_gpus < 1 || n_gpus > RT_MAX_GPUS) return fail(RT_ERR_INVALID, "n_gpus outside 1..16");
+    HostRender call;
+    if ((rc = call.begin(s, cfg)) != RT_OK) return rc;
+    const RenderJob& job = call.job;
+    const size_t npix = call.npix, n = call.n, nb = half_offset(n);
     if ((rc = ensure_adaptive_buffers(s, npix)) != RT_OK) return rc;
-    if (n_gpus > 1) {
-        if ((rc = ensure_replicas(s, n_gpus, 2 * nb)) != RT_OK) return rc; // d_accum = A | B, d_stage (no P2P route) as large
-        for (int g = 1; g < n_gpus; ++g) {
-            Replica& r = s->replicas[(size_t)g - 1];
-            if (npix <= r.list_cap) continue;
-            cudaError_t e;
-            if ((e = cudaSetDevice(r.device)) == cudaSuccess) {
-                if (r.d_list) cudaFree(r.d_list);
-                r.d_list = nullptr; r.list_cap = 0;
-                e = cudaMalloc(&r.d_list, npix * sizeof(uint32_t));
-            }
-            cudaSetDevice(s->dev.device);
-            if (e != cudaSuccess) return fail_cuda(e, "replica pixel list");
-            r.list_cap = npix;
-        }
-    }
+    if (n_gpus > 1 && (rc = ensure_replicas(s, n_gpus, 2 * nb, npix)) != RT_OK) return rc; // d_accum = A | B, d_stage (no P2P route) as large
     RenderBuffers& o = s->out;
     AdaptiveBuffers& b = s->adaptive;
-    const RenderTuning tune = tuning_for(s, cfg);
+    const RenderTuning tune = tuning_for_flags(s, cfg);
     const int32_t max = job.spp_total, step = ac->step;
     const uint32_t rendered = (uint32_t)job.width * (uint32_t)job.rows;
     cudaError_t e;
-    if ((e = cudaMemsetAsync(b.d_a, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess || (e = cudaMemsetAsync(b.d_b, 0, n * sizeof(int64_t), o.stream)) != cudaSuccess ||
+    if ((e = cudaMemsetAsync(b.d_ab, 0, 2 * nb * sizeof(int64_t), o.stream)) != cudaSuccess ||
         (e = cudaMemsetAsync(b.d_samples, 0, npix * sizeof(int32_t), o.stream)) != cudaSuccess || (e = launch_adaptive_iota(b.d_list[0], rendered, o.stream)) != cudaSuccess)
         return fail_cuda(e, "adaptive set-up");
 
-    // every GPU's A and B as GPU 0 reads them: in place (its own, P2P-mapped peers, alias mode) or copied into staging next to it
+    // every GPU's A and B as GPU 0 reads them
     auto shards = [&](AdaptiveShards& sh) -> cudaError_t {
         std::memset(&sh, 0, sizeof sh);
         sh.n = n_gpus;
-        sh.a[0] = b.d_a; sh.b[0] = b.d_b;
-        for (int g = 1; g < n_gpus; ++g) {
-            Replica& r = s->replicas[(size_t)g - 1];
-            const int64_t* ab = r.d_accum;
-            if (!r.peer_ok) {
-                const cudaError_t ce = cudaMemcpyPeerAsync(r.d_stage, s->dev.device, r.d_accum, r.device, 2 * nb * sizeof(int64_t), o.stream);
-                if (ce != cudaSuccess) return ce;
-                ab = r.d_stage;
-            }
-            sh.a[g] = ab; sh.b[g] = ab + nb;
-        }
-        return cudaSuccess;
+        const cudaError_t ce = gather_blocks(s, n_gpus, b.d_ab, 2 * nb, sh.a);
+        for (int g = 0; ce == cudaSuccess && g < n_gpus; ++g) sh.b[g] = sh.a[g] + nb;
+        return ce;
     };
 
     std::vector<std::vector<rt_stats>> st((size_t)n_gpus); // [GPU][round]
@@ -1812,16 +1811,16 @@ int32_t render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adapt
     std::vector<const char*> what((size_t)n_gpus, "");
     RoundBarrier bar(n_gpus - 1);
     uint32_t n_active = rendered; // written by GPU 0 at a check point, read by the workers once the barrier lets them go
-    int cur = 0;                  // GPU 0's current list (b.d_list[cur]); the workers' is r.d_list
+    int cur = 0;                  // GPU 0's current list (b.d_list[cur]); the workers' is their replica's d_list
     auto run = [&](int g) {
-        Replica* r = g ? &s->replicas[(size_t)g - 1] : nullptr;
-        cudaStream_t stream = r ? r->stream : o.stream;
-        int64_t* A = r ? r->d_accum : b.d_a;
-        int64_t* B = r ? r->d_accum + nb : b.d_b;
+        const GpuView v = gpu_view(s, g, b.d_ab);
+        int64_t* const A = v.accum;
+        int64_t* const B = v.accum + nb;
+        uint32_t* list = g ? s->replicas[(size_t)g - 1].d_list : b.d_list[cur];
         cudaError_t& err = errs[(size_t)g];
         auto stop = [&](cudaError_t ce, const char* w) { err = ce; what[(size_t)g] = w; bar.fail(); };
-        if (r && ((err = cudaSetDevice(r->device)) != cudaSuccess || (err = cudaMemsetAsync(r->d_accum, 0, 2 * nb * sizeof(int64_t), stream)) != cudaSuccess ||
-                  (err = launch_adaptive_iota(r->d_list, rendered, stream)) != cudaSuccess))
+        if (g > 0 && ((err = cudaSetDevice(v.device)) != cudaSuccess || (err = cudaMemsetAsync(v.accum, 0, 2 * nb * sizeof(int64_t), v.stream)) != cudaSuccess ||
+                      (err = launch_adaptive_iota(list, rendered, v.stream)) != cudaSuccess))
             return stop(err, "adaptive set-up");
         uint32_t na = rendered;
         for (int64_t k = 0; na > 0 && k * step < max; ++k) {
@@ -1829,7 +1828,7 @@ int32_t render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adapt
             const int32_t s0 = (int32_t)(k * step), s1 = (int32_t)std::min<int64_t>((k + 1) * step, max);
             RenderJob rj = job;
             rj.sample_begin = s0; rj.sample_end = s1;
-            rj.d_pixels = r ? r->d_list : b.d_list[cur]; rj.n_pixels = na;
+            rj.d_pixels = list; rj.n_pixels = na;
             // an even share of the round's paths: balanced in every round, consecutive paths on neighbouring pixels
             const uint64_t T = (uint64_t)na * (uint64_t)(s1 - s0);
             rj.path_begin = T * (uint64_t)g / (uint64_t)n_gpus;
@@ -1837,14 +1836,13 @@ int32_t render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adapt
             rt_stats rs;
             std::memset(&rs, 0, sizeof rs);
             if (rj.path_end > rj.path_begin) { // an empty range renders nothing (more GPUs than paths)
-                const DeviceScene& scene = r ? r->scene : s->dev.scene;
-                if ((err = launch_render(scene, rj, tune, (k & 1) ? B : A, stream, &rs, r ? &r->workspace : &s->workspace)) != cudaSuccess)
+                if ((err = launch_render(*v.scene, rj, tune, (k & 1) ? B : A, v.stream, &rs, v.workspace)) != cudaSuccess)
                     return stop(err, "adaptive render round");
             }
             st[(size_t)g].push_back(rs);
             if (!(k & 1) || s1 < ac->min_samples || s1 >= max) continue;
-            if (r) { // launch_render has drained the stream, except where the range was empty: the set-up may still be in flight
-                if ((err = cudaStreamSynchronize(stream)) != cudaSuccess) return stop(err, "adaptive round sync");
+            if (g > 0) { // launch_render has drained the stream, except where the range was empty: the set-up may still be in flight
+                if ((err = cudaStreamSynchronize(v.stream)) != cudaSuccess) return stop(err, "adaptive round sync");
                 if (!bar.arrive_and_wait()) return;
                 na = n_active;
                 continue;
@@ -1852,7 +1850,7 @@ int32_t render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adapt
             if (!bar.gather()) return;
             AdaptiveCheck c;
             if ((err = shards(c.shards)) != cudaSuccess) return stop(err, "peer copy");
-            c.d_list_in = b.d_list[cur]; c.n_active = na; c.d_list_out = b.d_list[cur ^ 1]; c.count_out = b.h_count;
+            c.d_list_in = list; c.n_active = na; c.d_list_out = b.d_list[cur ^ 1]; c.count_out = b.h_count;
             c.d_u = b.d_u; c.d_keep = b.d_keep; c.d_samples = b.d_samples;
             c.d_temp = b.d_temp; c.temp_bytes = b.temp_bytes;
             c.W = job.width; c.rows = job.rows; c.n = s1; c.radius = ac->radius; c.threshold = ac->threshold;
@@ -1860,53 +1858,35 @@ int32_t render_adaptive(rt_scene* s, const rt_render_config* cfg, const rt_adapt
             if ((err = cudaStreamSynchronize(o.stream)) != cudaSuccess) return stop(err, "adaptive check sync");
             na = n_active = *b.h_count;
             cur ^= 1;
+            list = b.d_list[cur];
             if (n_gpus > 1) {
                 for (int h = 1; h < n_gpus && na > 0; ++h) {
                     Replica& rh = s->replicas[(size_t)h - 1];
-                    if ((err = cudaMemcpyPeerAsync(rh.d_list, rh.device, b.d_list[cur], s->dev.device, na * sizeof(uint32_t), o.stream)) != cudaSuccess)
+                    if ((err = cudaMemcpyPeerAsync(rh.d_list, rh.device, list, s->dev.device, na * sizeof(uint32_t), o.stream)) != cudaSuccess)
                         return stop(err, "pixel list copy");
                 }
                 if ((err = cudaStreamSynchronize(o.stream)) != cudaSuccess) return stop(err, "pixel list copy sync");
                 bar.release();
             }
         }
-        if (r && (err = cudaStreamSynchronize(stream)) != cudaSuccess) return stop(err, "adaptive round sync");
+        if (g > 0 && (err = cudaStreamSynchronize(v.stream)) != cudaSuccess) return stop(err, "adaptive round sync");
     };
-    {
-        std::vector<std::thread> pool;
-        bool started = true;
-        try {
-            for (int g = 1; g < n_gpus; ++g) pool.emplace_back(run, g);
-        } catch (const std::system_error&) {
-            started = false;
-            bar.fail();
-        }
-        if (started) run(0); // the calling thread is GPU 0
-        for (std::thread& th : pool) th.join();
-        if (!started) return fail(RT_ERR_CUDA, "could not start the render threads");
-    }
+    if ((rc = run_on_gpus(n_gpus, run, [&] { bar.fail(); })) != RT_OK) return rc;
     for (int g = 0; g < n_gpus; ++g)
         if (errs[(size_t)g] != cudaSuccess) return fail_cuda(errs[(size_t)g], what[(size_t)g]);
     AdaptiveShards sh;
     if ((e = launch_adaptive_fill(b.d_list[cur], n_active, max, b.d_samples, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive counts");
     if ((e = shards(sh)) != cudaSuccess) return fail_cuda(e, "peer copy");
     if ((e = launch_resolve_adaptive(sh, b.d_samples, o.d_accum, o.d_u8, job.width, job.height, o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive resolve");
-    if (out_screen && (e = cudaMemcpyAsync(o.h_u8, o.d_u8, n, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "screen copy");
-    if (out_accum && (e = cudaMemcpyAsync(out_accum, o.d_accum, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "accum copy");
-    if (out_samples && (e = cudaMemcpyAsync(out_samples, b.d_samples, npix * sizeof(int32_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
-        return fail_cuda(e, "samples copy");
-    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "adaptive sync");
-    if (out_screen) widen_screen(o.h_u8, out_screen, n);
-    if (stats) { // the GPUs of a round run at the same time, the rounds one after the other
-        std::memset(stats, 0, sizeof *stats);
-        for (size_t k = 0; k < st[0].size(); ++k) {
-            rt_stats round = st[0][k];
-            for (int g = 1; g < n_gpus; ++g) add_stats(round, st[(size_t)g][k], true);
-            add_stats(*stats, round, false);
-        }
-        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    rt_stats sum; // the GPUs of a round run at the same time, the rounds one after the other
+    std::memset(&sum, 0, sizeof sum);
+    for (size_t k = 0; k < st[0].size(); ++k) {
+        rt_stats round = st[0][k];
+        for (int g = 1; g < n_gpus; ++g) add_stats(round, st[(size_t)g][k], true);
+        add_stats(sum, round, false);
     }
-    return RT_OK;
+    return call.finish(out_screen, {{out_accum, o.d_accum, n * sizeof(int64_t), "accum copy"}, {out_samples, b.d_samples, npix * sizeof(int32_t), "samples copy"}},
+                       "adaptive sync", sum, stats);
 }
 
 } // namespace
@@ -1962,31 +1942,17 @@ int32_t aov_pass(rt_scene* s, const RenderJob& job, cudaStream_t stream, rt_stat
 int32_t RTB_FN(render_aov)(rt_scene* s, const rt_render_config* cfg, int64_t* out_albedo, int64_t* out_normal, rt_stats* stats) {
     CHECK_SCENE(s);
     if (!cfg) return fail(RT_ERR_INVALID, "null config");
-    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
-        return fail(RT_ERR_INVALID, "rt_render_aov takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
-    RenderJob job;
-    int32_t rc = make_job(s, cfg, job);
+    int32_t rc = check_whole_render(cfg, "rt_render_aov", false);
     if (rc != RT_OK) return rc;
-    const auto t0 = std::chrono::steady_clock::now();
-    DeviceGuard guard(s->dev.device);
-    const size_t npix = (size_t)job.width * job.height, n = npix * 3;
-    if ((rc = ensure_out_buffers(s, n)) != RT_OK) return rc;
-    if ((rc = ensure_denoise_buffers(s, npix)) != RT_OK) return rc;
-    RenderBuffers& o = s->out;
+    HostRender call;
+    if ((rc = call.begin(s, cfg)) != RT_OK) return rc;
+    if ((rc = ensure_denoise_buffers(s, call.npix)) != RT_OK) return rc;
     rt_stats st;
     std::memset(&st, 0, sizeof st);
-    if ((rc = aov_pass(s, job, o.stream, &st)) != RT_OK) return rc;
-    cudaError_t e;
-    if (out_albedo && (e = cudaMemcpyAsync(out_albedo, s->denoise.d_albedo, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
-        return fail_cuda(e, "albedo copy");
-    if (out_normal && (e = cudaMemcpyAsync(out_normal, s->denoise.d_normal, n * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
-        return fail_cuda(e, "normal copy");
-    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "feature sync");
-    if (stats) {
-        *stats = st;
-        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    }
-    return RT_OK;
+    if ((rc = aov_pass(s, call.job, s->out.stream, &st)) != RT_OK) return rc;
+    const size_t bytes = call.n * sizeof(int64_t);
+    return call.finish(nullptr, {{out_albedo, s->denoise.d_albedo, bytes, "albedo copy"}, {out_normal, s->denoise.d_normal, bytes, "normal copy"}}, "feature sync",
+                       st, stats);
 }
 
 int32_t rt_render_denoised(rt_scene* s, const rt_render_config* cfg, const rt_denoise_config* dc, double* out_screen, double* out_linear,
@@ -2001,27 +1967,22 @@ int32_t rt_render_denoised(rt_scene* s, const rt_render_config* cfg, const rt_de
     if (dc->iterations < 1 || dc->iterations > 8) return fail(RT_ERR_INVALID, "denoise iterations outside 1..8");
     for (double sg : {dc->sigma_color, dc->sigma_albedo, dc->sigma_normal})
         if (!(sg > 0.0) || !std::isfinite(sg)) return fail(RT_ERR_INVALID, "denoise sigmas must be finite and > 0");
-    if (RT_RENDER_TILE_COUNT(cfg->flags) > 1 || (cfg->flags & RT_RENDER_NO_WAIT))
-        return fail(RT_ERR_INVALID, "rt_render_denoised takes neither a tile shard (RT_RENDER_TILE_SHARD with count > 1) nor RT_RENDER_NO_WAIT");
-    if (cfg->sample_begin != 0 || (cfg->sample_end != 0 && cfg->sample_end != n))
-        return fail(RT_ERR_INVALID, "rt_render_denoised renders every sample range itself: sample_begin / sample_end must cover [0, samples_per_pixel)");
-    RenderJob job;
-    int32_t rc = make_job(s, cfg, job);
+    int32_t rc = check_whole_render(cfg, "rt_render_denoised", true);
     if (rc != RT_OK) return rc;
-    const auto t0 = std::chrono::steady_clock::now();
-    DeviceGuard guard(s->dev.device);
-    const size_t npix = (size_t)job.width * job.height, n3 = npix * 3;
-    if ((rc = ensure_out_buffers(s, n3)) != RT_OK) return rc;
+    HostRender call;
+    if ((rc = call.begin(s, cfg)) != RT_OK) return rc;
+    const RenderJob& job = call.job;
+    const size_t npix = call.npix, n3 = call.n, nb = half_offset(n3);
     if ((rc = ensure_adaptive_buffers(s, npix)) != RT_OK) return rc;
     if ((rc = ensure_denoise_buffers(s, npix)) != RT_OK) return rc;
     RenderBuffers& o = s->out;
-    AdaptiveBuffers& ab = s->adaptive;
     DenoiseBuffers& db = s->denoise;
-    const RenderTuning tune = tuning_for(s, cfg);
+    int64_t* const A = s->adaptive.d_ab;
+    int64_t* const B = A + nb;
+    const RenderTuning tune = tuning_for_flags(s, cfg);
     const int32_t hA = n / 2;
     cudaError_t e;
-    if ((e = cudaMemsetAsync(ab.d_a, 0, n3 * sizeof(int64_t), o.stream)) != cudaSuccess || (e = cudaMemsetAsync(ab.d_b, 0, n3 * sizeof(int64_t), o.stream)) != cudaSuccess)
-        return fail_cuda(e, "denoise set-up");
+    if ((e = cudaMemsetAsync(A, 0, 2 * nb * sizeof(int64_t), o.stream)) != cudaSuccess) return fail_cuda(e, "denoise set-up");
     rt_stats sum;
     std::memset(&sum, 0, sizeof sum);
     // the two half renders: samples [0, hA) into A and [hA, n) into B (their sum is rt_render's accumulator bit for bit)
@@ -2031,7 +1992,7 @@ int32_t rt_render_denoised(rt_scene* s, const rt_render_config* cfg, const rt_de
         hj.sample_end = half ? n : hA;
         rt_stats rs;
         std::memset(&rs, 0, sizeof rs);
-        if ((e = launch_render(s->dev.scene, hj, tune, half ? ab.d_b : ab.d_a, o.stream, &rs, &s->workspace)) != cudaSuccess) return fail_cuda(e, "denoise half render");
+        if ((e = launch_render(s->dev.scene, hj, tune, half ? B : A, o.stream, &rs, &s->workspace)) != cudaSuccess) return fail_cuda(e, "denoise half render");
         add_stats(sum, rs, false);
     }
     RenderJob aj = job;
@@ -2042,25 +2003,15 @@ int32_t rt_render_denoised(rt_scene* s, const rt_render_config* cfg, const rt_de
     if ((rc = aov_pass(s, aj, o.stream, &as)) != RT_OK) return rc;
     sum.kernel_launches += as.kernel_launches;
     DenoiseJob dj;
-    dj.a = ab.d_a; dj.b = ab.d_b; dj.albedo = db.d_albedo; dj.normal = db.d_normal;
+    dj.a = A; dj.b = B; dj.albedo = db.d_albedo; dj.normal = db.d_normal;
     dj.W = job.width; dj.H = job.height; dj.rows = job.rows; dj.hA = hA; dj.hB = n - hA; dj.m = dc->aov_samples; dj.iterations = dc->iterations;
     dj.sigma_color = dc->sigma_color; dj.sigma_albedo = dc->sigma_albedo; dj.sigma_normal = dc->sigma_normal;
     dj.c[0] = db.d_c[0]; dj.c[1] = db.d_c[1]; dj.v[0] = db.d_v[0]; dj.v[1] = db.d_v[1]; dj.vbar = db.d_vbar; dj.feat = db.d_feat;
     dj.accum_out = o.d_accum; dj.linear_out = db.d_linear; dj.screen_u8 = o.d_u8;
     if ((e = launch_denoise(dj, o.stream)) != cudaSuccess) return fail_cuda(e, "denoise filter");
     sum.kernel_launches += 2 + 2 * (uint64_t)dc->iterations;
-    if (out_screen && (e = cudaMemcpyAsync(o.h_u8, o.d_u8, n3, cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess) return fail_cuda(e, "screen copy");
-    if (out_linear && (e = cudaMemcpyAsync(out_linear, db.d_linear, n3 * sizeof(double), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
-        return fail_cuda(e, "linear copy");
-    if (out_accum && (e = cudaMemcpyAsync(out_accum, o.d_accum, n3 * sizeof(int64_t), cudaMemcpyDeviceToHost, o.stream)) != cudaSuccess)
-        return fail_cuda(e, "accum copy");
-    if ((e = cudaStreamSynchronize(o.stream)) != cudaSuccess) return fail_cuda(e, "denoise sync");
-    if (out_screen) widen_screen(o.h_u8, out_screen, n3);
-    if (stats) {
-        *stats = sum;
-        stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    }
-    return RT_OK;
+    return call.finish(out_screen, {{out_linear, db.d_linear, n3 * sizeof(double), "linear copy"}, {out_accum, o.d_accum, n3 * sizeof(int64_t), "accum copy"}},
+                       "denoise sync", sum, stats);
 }
 
 // ---- peer group: the exchange of the one-process-per-GPU layout without a collective library on the data path
